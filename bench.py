@@ -2,7 +2,7 @@
 """Benchmark of the hot path: from-scratch control matrix -> filter function -> infidelity.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload d4|c2|c3] [--extra c2,c3|none]
-                    [--impl reference]
+                    [--impl reference] [--dump-outputs DIR]
 
 A *step* is one pass of the whole path over one synthetic pulse (SURVEY.md 8d): diagonalise the
 G-segment control Hamiltonian, build the first-order control matrix on n_omega frequencies, reduce it
@@ -26,6 +26,11 @@ BASELINE.json's: control-matrix throughput in segment*frequency pairs per second
           same pulse, all frequencies; the reference's cost is exactly linear in G) -- the printed
           ms_per_step is EXTRAPOLATED to the full pulse.  Falls back to the NumPy port in oracle/ if
           the reference has not been staged.
+  --dump-outputs DIR : after the timed steps, write what the last timed step of the headline workload
+          computed (device path: eigenvalues, eigenvectors, propagators, control matrix, filter function,
+          infidelities; public API: its infidelities) as DIR/<name>.npy, so that the outputs of two builds
+          can be compared on identical (seeded) inputs.  With N > 1 the frequency-resolved arrays are rank
+          0's block of the grid.
 """
 import argparse
 import json
@@ -74,7 +79,17 @@ def parse_args():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-int8', action='store_true',
                     help="skip the extra 'd4_int8' line (opt-in int8 tensor-core kernel)")
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step of the headline workload as '
+                         'DIR/<name>.npy (float64, complex arrays with a trailing (real, imag) axis, at '
+                         'most 64 MB in all: larger frequency-resolved arrays keep a fixed, seeded sample '
+                         'of frequencies)')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs is not None and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of the GPU path (--impl b200)')
+    return args
 
 
 def workload_config(wl, n_gpus, n_local):
@@ -313,22 +328,50 @@ def kernel_model(wl, n_omega_local, kernel_ms, peak, int8=False):
     return kernel, pipe, executed, executed
 
 
-def measure(name, steps, warmup, env, int8=False):
+def measure(name, steps, warmup, env, int8=False, dump=False):
     """One workload on this rank's GPU: device-resident value, e2e through the public API, roofline of
     the control-matrix kernel.  Collective over the ranks (every rank calls it with the same name).
     ``int8``: with the opt-in fixed-point control-matrix kernel on the int8 tensor cores
-    (FFB_CTRLMAT_INT8=1, d = 4 only)."""
+    (FFB_CTRLMAT_INT8=1, d = 4 only).  ``dump``: the result also holds, under 'outputs', host copies
+    of what the last timed step computed."""
     if int8:
         old = os.environ.get('FFB_CTRLMAT_INT8')
         os.environ['FFB_CTRLMAT_INT8'] = '1'
         try:
-            return _measure(name, steps, warmup, env, True)
+            return _measure(name, steps, warmup, env, True, dump)
         finally:
             if old is None:
                 os.environ.pop('FFB_CTRLMAT_INT8', None)
             else:
                 os.environ['FFB_CTRLMAT_INT8'] = old
-    return _measure(name, steps, warmup, env, os.environ.get('FFB_CTRLMAT_INT8', '0') not in ('', '0'))
+    return _measure(name, steps, warmup, env, os.environ.get('FFB_CTRLMAT_INT8', '0') not in ('', '0'),
+                    dump)
+
+
+DUMP_BYTES = 64_000_000
+FREQUENCY_RESOLVED = ('control_matrix', 'filter_function')
+
+
+def dump_outputs(directory, outputs):
+    """Write ``outputs`` (name -> array) as ``directory/<name>.npy`` in float64, a complex array with a
+    trailing axis (real, imag).  If the files would exceed DUMP_BYTES, the frequency-resolved arrays keep
+    the same fixed, seeded sample of their frequencies (last axis), identical from run to run."""
+    n_omega = outputs['control_matrix'].shape[-1]
+    budget = DUMP_BYTES - 1024*len(outputs)     # room for the .npy headers
+    total = sum(a.nbytes for a in outputs.values())
+    if total > budget:
+        per_omega = sum(outputs[k].nbytes for k in FREQUENCY_RESOLVED)//n_omega
+        n_keep = (budget - (total - per_omega*n_omega))//per_omega
+        if n_keep < 1:
+            raise SystemExit(f'--dump-outputs: the arrays that do not depend on frequency alone exceed '
+                             f'{DUMP_BYTES} bytes')
+        keep =np.sort(np.random.default_rng(0).choice(n_omega, n_keep, replace=False))
+        outputs = {k: a[..., keep] if k in FREQUENCY_RESOLVED else a for k, a in outputs.items()}
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        if np.iscomplexobj(a):
+            a = np.stack([a.real, a.imag], axis=-1)
+        np.save(os.path.join(directory, f'{name}.npy'), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def control_matrix_parity(name, B):
@@ -343,7 +386,7 @@ def control_matrix_parity(name, B):
                      for j in range(len(B))))
 
 
-def _measure(name, steps, warmup, env, int8):
+def _measure(name, steps, warmup, env, int8, dump):
     import ctypes
 
     import torch
@@ -402,6 +445,11 @@ def _measure(name, steps, warmup, env, int8):
     _lib.check(ctx, L.ffb_kernel_timing_enable(ctx, 0))
     dev_ms = sum(e0.elapsed_time(e1) for e0, e1 in events)
     dev_inf = (total if (world > 1 and peers is None) else dev.infidelity).cpu().numpy()
+    outputs = None
+    if dump:    # what a caller of DevicePulse.step() holds after the last timed step
+        outputs = {k: getattr(dev, k).cpu().numpy() for k in
+                   ('eigvals', 'eigvecs', 'propagators', 'control_matrix', 'filter_function')}
+        outputs['infidelity'] = dev_inf
     if peers is not None:
         _lib.check(ctx, L.ffb_comm_reduce_infidelity(ctx, 0))
 
@@ -453,6 +501,8 @@ def _measure(name, steps, warmup, env, int8):
     order = np.argsort(wl.n_ids)           # PulseSequence sorts operators by identifier
     dev_inf = dev_inf[order]
     api = np.asarray(infid_e2e).ravel()
+    if dump:
+        outputs['e2e_infidelity'] = np.asarray(infid_e2e)
     parity = {'device_vs_api': float(np.abs(dev_inf - api).max()/np.abs(api).max()),
               'vs_reference_fixture': golden_parity(name, order, api),
               'tolerance': 1e-10}
@@ -504,7 +554,7 @@ def _measure(name, steps, warmup, env, int8):
                         else 'filter_functions_b200.distributed.infidelity(PulseSequence, spectrum, '
                              'omega) on a cold cache, global grid, every rank')},
         'gpu_launches': int(launches), 'roofline': roofline, 'parity': parity,
-        'infidelity': api.tolist()[:6],
+        'infidelity': api.tolist()[:6], **({'outputs': outputs} if dump else {}),
     }
 
 
@@ -552,7 +602,7 @@ def run_b200(args):
                peak_source='measured live by ffb_measure_fp64_peak (DFMA %.2f, DMMA %.2f TFLOP/s); '
                            'MEASURED_PEAKS.json has no fp64 entry' % (dfma.value, dmma.value))
 
-    head = measure(args.workload, args.steps, args.warmup, env)
+    head = measure(args.workload, args.steps, args.warmup, env, dump=args.dump_outputs is not None)
     if args.extra is None:
         extra = [w for w in ('c2', 'c3', 'd4') if w != args.workload]
     else:
@@ -574,6 +624,8 @@ def run_b200(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, head['outputs'])
 
     cpu = None
     if not args.no_cpu_baseline and world == 1:

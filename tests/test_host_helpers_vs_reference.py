@@ -1,10 +1,10 @@
 """Differential test (CPU) of the host helpers that were added for drop-in completeness against the
-UNMODIFIED reference staged under ``baseline/_ref`` (skipped where it is not staged): ``util.tensor``,
-``util.remove_float_errors``, ``Basis.from_partial`` / ``pauli`` / ``ggm`` / expansions and predicates,
-``superoperator.liouville_to_choi`` / ``liouville_is_CP`` / ``liouville_is_cCP``, ``util.get_sample_frequencies``,
-``util.parse_operators`` / ``parse_spectrum`` error behaviour.  None of these needs the GPU."""
-import os
-import sys
+UNMODIFIED reference: ``util.tensor``, ``util.remove_float_errors``, ``Basis.from_partial`` / ``pauli`` /
+``ggm`` / expansions and predicates, ``superoperator.liouville_to_choi`` / ``liouville_is_CP`` /
+``liouville_is_cCP``, ``util.get_sample_frequencies``, ``util.parse_operators`` / ``parse_spectrum`` error
+behaviour.  The reference runs where it is staged under ``baseline/_ref``; elsewhere its results on these
+seeded inputs come from ``tests/golden/reference_host_helpers.pkl.gz`` (``helpers.ReferenceResults``).  None
+of these needs the GPU."""
 import warnings
 
 import numpy as np
@@ -12,20 +12,14 @@ import pytest
 
 import filter_functions_b200 as ffb
 from filter_functions_b200 import superoperator as so_new
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, 'baseline', '_ref')
+from helpers import RAISED, ReferenceResults
 
 
 @pytest.fixture(scope='module')
 def ref():
-    if not os.path.isdir(os.path.join(REF, 'filter_functions')):
-        pytest.skip('reference not staged under baseline/_ref')
-    for p in (os.path.join(ROOT, 'oracle', 'shim'), REF):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    import filter_functions
-    return filter_functions
+    results = ReferenceResults('reference_host_helpers')
+    yield results
+    results.save()
 
 
 def herm(rng, d, n=1):
@@ -33,9 +27,15 @@ def herm(rng, d, n=1):
     return a + a.conj().swapaxes(1, 2)
 
 
+def basis_data(b):
+    return {'array': b.view(np.ndarray).copy(), 'labels': list(b.labels), 'btype': b.btype,
+            **{pred: bool(getattr(b, pred)) for pred in
+               ('isherm', 'isnorm', 'isorthogonal', 'isorthonorm', 'istraceless', 'iscomplete')}}
+
+
 def test_tensor_and_cleanup(ref):
     rng = np.random.default_rng(0)
-    for _ in range(60):
+    for case in range(60):
         rank = int(rng.integers(1, 4))
         n_args = int(rng.integers(1, 4))
         lead = tuple(rng.integers(1, 4, size=rng.integers(0, 3)))
@@ -44,35 +44,38 @@ def test_tensor_and_cleanup(ref):
             shape = tuple(rng.integers(1, 4, size=rank))
             my_lead = tuple(1 if rng.random() < 0.3 else n for n in lead)[rng.integers(0, len(lead) + 1):]
             args.append(rng.standard_normal(my_lead + shape) + 1j*rng.standard_normal(my_lead + shape))
-        try:
-            want = ref.util.tensor(*args, rank=rank)
-        except ValueError as err:
+        want = ref(f'tensor/{case}', lambda m: m.util.tensor(*args, rank=rank))
+        if isinstance(want, tuple) and want[0] == RAISED:
             with pytest.raises(ValueError) as got:
                 ffb.util.tensor(*args, rank=rank)
-            assert str(got.value) == str(err)
+            assert str(got.value) == want[1]
             continue
         got = ffb.util.tensor(*args, rank=rank)
         assert got.shape == want.shape and np.allclose(got, want, rtol=1e-14, atol=0)
     for dtype in (float, complex):
         x = (np.eye(4) + 1e-17*rng.standard_normal((4, 4))).astype(dtype)
-        assert np.array_equal(ffb.util.remove_float_errors(x.copy()), ref.util.remove_float_errors(x.copy()))
-        assert np.array_equal(ffb.util.remove_float_errors(x.copy(), 100), ref.util.remove_float_errors(x.copy(), 100))
+        for args in ((), (100,)):
+            want = ref(f'remove_float_errors/{dtype.__name__}/{args}',
+                       lambda m: m.util.remove_float_errors(x.copy(), *args))
+            assert np.array_equal(ffb.util.remove_float_errors(x.copy(), *args), want)
 
 
 def test_basis_constructors_predicates_and_expansion(ref):
     rng = np.random.default_rng(1)
     for n in (1, 2):
-        assert np.array_equal(ffb.Basis.pauli(n), ref.Basis.pauli(n).view(np.ndarray))
-        assert list(ffb.Basis.pauli(n).labels) == list(ref.Basis.pauli(n).labels)
+        want = ref(f'pauli/{n}', lambda m: basis_data(m.Basis.pauli(n)))
+        assert np.array_equal(ffb.Basis.pauli(n), want['array'])
+        assert list(ffb.Basis.pauli(n).labels) == want['labels']
     for d in (2, 3, 4, 5):
-        a, b = ffb.Basis.ggm(d), ref.Basis.ggm(d)
-        assert np.allclose(a.view(np.ndarray), b.view(np.ndarray), atol=1e-16)
-        assert list(a.labels) == list(b.labels) and a.btype == b.btype
+        a, b = ffb.Basis.ggm(d), ref(f'ggm/{d}', lambda m: basis_data(m.Basis.ggm(d)))
+        assert np.allclose(a.view(np.ndarray), b['array'], atol=1e-16)
+        assert list(a.labels) == b['labels'] and a.btype == b['btype']
         M = herm(rng, d, 3)
         for kw in (dict(), dict(hermitian=True), dict(traceless=True), dict(tidyup=True)):
-            assert np.allclose(a.expand(M, **kw), b.expand(M, **kw), atol=1e-14)
+            want = ref(f'ggm/{d}/expand/{sorted(kw)}', lambda m: m.Basis.ggm(d).expand(M, **kw))
+            assert np.allclose(a.expand(M, **kw), want, atol=1e-14)
         # partial bases: random orthogonal subsets in a rotated frame, with and without the identity
-        g = b.view(np.ndarray)
+        g = b['array']
         for trial in range(6):
             n = int(rng.integers(1, d*d))
             q, _ = np.linalg.qr(rng.standard_normal((d*d, d*d)))
@@ -80,42 +83,49 @@ def test_basis_constructors_predicates_and_expansion(ref):
                     else g[rng.choice(d*d, size=n, replace=False)]*rng.uniform(0.5, 3))
             with warnings.catch_warnings():
                 warnings.simplefilter('ignore')
-                want, got = ref.Basis.from_partial(part), ffb.Basis.from_partial(part)
-            assert got.shape == want.shape and got.btype == want.btype and list(got.labels) == list(want.labels)
+                want = ref(f'from_partial/{d}/{trial}', lambda m: basis_data(m.Basis.from_partial(part)))
+                got = ffb.Basis.from_partial(part)
+            assert got.shape == want['array'].shape and got.btype == want['btype']
+            assert list(got.labels) == want['labels']
             for pred in ('isherm', 'isnorm', 'isorthogonal', 'isorthonorm', 'istraceless', 'iscomplete'):
-                assert bool(getattr(got, pred)) == bool(getattr(want, pred)), pred
+                assert bool(getattr(got, pred)) == want[pred], pred
             # both are complete orthonormal bases (the map between them is unitary) and the given elements
             # (plus the identity of a traceless basis) sit at the same positions in both
-            gw, gg = want.view(np.ndarray).reshape(d*d, -1), got.view(np.ndarray).reshape(d*d, -1)
+            gw, gg = want['array'].reshape(d*d, -1), got.view(np.ndarray).reshape(d*d, -1)
             overlap = gw.conj() @ gg.T
             assert np.allclose(np.abs(np.linalg.det(overlap)), 1, atol=1e-9)
             same = [i for i in range(d*d) if np.isclose(abs(overlap[i, i]), 1, atol=1e-9)]
             assert len(same) >= n
     X, Y = ffb.util.paulis[1:3]
-    for args, kw in (([X, X + Y], {}), ([np.diag([1.0, 0])], dict(traceless=True)), ([X, Y], dict(labels=['a']))):
-        with pytest.raises(ValueError) as e_ref:
-            ref.Basis.from_partial(args, **kw)
+    for case, (args, kw) in enumerate((([X, X + Y], {}), ([np.diag([1.0, 0])], dict(traceless=True)),
+                                       ([X, Y], dict(labels=['a'])))):
+        want = ref(f'from_partial/error/{case}', lambda m: basis_data(m.Basis.from_partial(args, **kw)))
+        assert isinstance(want, tuple) and want[0] == RAISED
         with pytest.raises(ValueError) as e_new:
             ffb.Basis.from_partial(args, **kw)
-        assert str(e_new.value) == str(e_ref.value)
+        assert str(e_new.value) == want[1]
 
 
 def test_choi_and_cp_checks(ref):
     rng = np.random.default_rng(2)
     for d in (2, 3, 4):
-        b_ref, b_new = ref.Basis.ggm(d), ffb.Basis.ggm(d)
+        b_new = ffb.Basis.ggm(d)
         S = rng.standard_normal((4, d*d, d*d)) + 1j*rng.standard_normal((4, d*d, d*d))
-        assert np.allclose(so_new.liouville_to_choi(S, b_new), ref.superoperator.liouville_to_choi(S, b_ref))
+        want = ref(f'choi/{d}', lambda m: m.superoperator.liouville_to_choi(S, m.Basis.ggm(d)))
+        assert np.allclose(so_new.liouville_to_choi(S, b_new), want)
         H = herm(rng, d)[0]
         w, v = np.linalg.eigh(H)
         U = (v*np.exp(-1j*w)) @ v.conj().T
-        L = ref.superoperator.liouville_representation(U, b_ref)
+        L = ref(f'liouville/{d}', lambda m: m.superoperator.liouville_representation(U, m.Basis.ggm(d)))
         for fn in ('liouville_is_CP', 'liouville_is_cCP'):
-            for arg in (L, -L, S, np.stack([L, -np.eye(d*d)])):
-                want = getattr(ref.superoperator, fn)(arg, b_ref, return_eig=True)
+            for i, arg in enumerate((L, -L, S, np.stack([L, -np.eye(d*d)]))):
+                def call(m):
+                    res = getattr(m.superoperator, fn)(arg, m.Basis.ggm(d), return_eig=True)
+                    return np.asarray(res[0]), np.asarray(res[1][0])
+                want = ref(f'{fn}/{d}/{i}', call)
                 got = getattr(so_new, fn)(arg, b_new, return_eig=True)
-                assert np.array_equal(np.asarray(got[0]), np.asarray(want[0])), fn
-                assert np.allclose(got[1][0], want[1][0], atol=1e-10)
+                assert np.array_equal(np.asarray(got[0]), want[0]), fn
+                assert np.allclose(got[1][0], want[1], atol=1e-10)
 
 
 def test_sample_frequencies_and_parsers(ref):
@@ -124,21 +134,24 @@ def test_sample_frequencies_and_parsers(ref):
     for G in (1, 5, 40):
         dt = rng.uniform(0.1, 2, G)
         coeffs = rng.standard_normal(G)
-        a = ref.PulseSequence([[X/2, coeffs, 'X']], [[Z/2, np.ones(G), 'Z']], dt)
         b = ffb.PulseSequence([[X/2, coeffs, 'X']], [[Z/2, np.ones(G), 'Z']], dt)
-        for kw in (dict(), dict(n_samples=57, spacing='linear'), dict(include_quasistatic=True),
-                   dict(omega_min=1e-3, omega_max=7.0)):
-            assert np.array_equal(ffb.util.get_sample_frequencies(b, **kw), ref.util.get_sample_frequencies(a, **kw))
+        for i, kw in enumerate((dict(), dict(n_samples=57, spacing='linear'), dict(include_quasistatic=True),
+                                dict(omega_min=1e-3, omega_max=7.0))):
+            want = ref(f'sample_frequencies/{G}/{i}', lambda m: m.util.get_sample_frequencies(
+                m.PulseSequence([[X/2, coeffs, 'X']], [[Z/2, np.ones(G), 'Z']], dt), **kw))
+            assert np.array_equal(ffb.util.get_sample_frequencies(b, **kw), want)
         with pytest.raises(ValueError):
             ffb.util.get_sample_frequencies(b, spacing='foo')
     omega = np.linspace(0, 1, 11)
-    for S, idx in ((np.ones((2, 11)), [0, 1]), (np.ones(11), [0]), (np.ones((2, 2, 11)) + 0j, [0, 1])):
-        assert np.array_equal(ffb.util.parse_spectrum(S, omega, np.array(idx)), ref.util.parse_spectrum(S, omega, np.array(idx)))
+    for i, (S, idx) in enumerate(((np.ones((2, 11)), [0, 1]), (np.ones(11), [0]),
+                                  (np.ones((2, 2, 11)) + 0j, [0, 1]))):
+        want = ref(f'parse_spectrum/{i}', lambda m: m.util.parse_spectrum(S, omega, np.array(idx)))
+        assert np.array_equal(ffb.util.parse_spectrum(S, omega, np.array(idx)), want)
     bad = [(np.ones((3, 11)), [0, 1]), (np.ones((2, 2, 2, 11)), [0, 1]), (np.ones(10), [0]),
            (np.arange(44).reshape(2, 2, 11)*(1 + 1j), [0, 1])]
-    for S, idx in bad:
-        with pytest.raises(ValueError) as e_ref:
-            ref.util.parse_spectrum(S, omega, np.array(idx))
+    for i, (S, idx) in enumerate(bad):
+        want = ref(f'parse_spectrum/error/{i}', lambda m: m.util.parse_spectrum(S, omega, np.array(idx)))
+        assert isinstance(want, tuple) and want[0] == RAISED
         with pytest.raises(ValueError) as e_new:
             ffb.util.parse_spectrum(S, omega, np.array(idx))
-        assert str(e_new.value) == str(e_ref.value)
+        assert str(e_new.value) == want[1]

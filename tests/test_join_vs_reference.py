@@ -1,28 +1,21 @@
 """Differential test of the Hamiltonian join (``concatenate_without_filter_function``, reference
 ``pulse_sequence.py:1340-1483, :1599-1665``) against the UNMODIFIED reference staged under
-``baseline/_ref`` (skipped where it is not staged): random pulse libraries with shared / partially
-shared operators, identifier clashes, equal operators under different identifiers and non-constant
-noise sensitivities; results, identifier mappings and exception types + messages must agree.  Every
-library is joined in several random orders, so that the remembered join plans are exercised."""
-import importlib.util
-import os
-import sys
-
+``baseline/_ref`` where it is staged, elsewhere against its results on these seeded inputs stored in
+``tests/golden/reference_join.pkl.gz`` (``helpers.ReferenceResults``): random pulse libraries with shared /
+partially shared operators, identifier clashes, equal operators under different identifiers and
+non-constant noise sensitivities; results, identifier mappings and exception types + messages must agree.
+Every library is joined in several random orders, so that the remembered join plans are exercised."""
 import numpy as np
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, 'baseline', '_ref')
+from helpers import ReferenceResults
 
 
-def load_reference():
-    if not os.path.isdir(os.path.join(REF, 'filter_functions')):
-        pytest.skip('reference not staged under baseline/_ref')
-    for p in (os.path.join(ROOT, 'oracle', 'shim'), REF):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    import filter_functions
-    return filter_functions
+@pytest.fixture(scope='module')
+def ref():
+    results = ReferenceResults('reference_join')
+    yield results
+    results.save()
 
 
 X = np.array([[0, 1], [1, 0]], dtype=complex)
@@ -54,7 +47,7 @@ def random_library(rng, n_lib, nasty):
     return recipes
 
 
-def outcome(package, join, pulses):
+def outcome(join, pulses):
     try:
         new, cmap, nmap = join(pulses, return_identifier_mappings=True)
     except Exception as err:        # noqa: BLE001 -- the type and text are what is compared
@@ -64,24 +57,25 @@ def outcome(package, join, pulses):
             {int(k): dict(v) for k, v in cmap.items()}, {int(k): dict(v) for k, v in nmap.items()})
 
 
+def joined(package, recipes, idx):
+    pulses = [package.PulseSequence(c, n, dt) for c, n, dt in recipes]
+    return outcome(package.pulse_sequence.concatenate_without_filter_function, [pulses[i] for i in idx])
+
+
 @pytest.mark.parametrize('nasty', [False, True])
-def test_join_matches_reference(nasty):
-    ref = load_reference()
+def test_join_matches_reference(ref, nasty):
     import filter_functions_b200 as ff
     rng = np.random.default_rng(2026 + nasty)
     n_ok = n_err = 0
-    for _ in range(60):
+    for lib in range(60):
         recipes = random_library(rng, int(rng.integers(2, 7)), nasty)
         if len(recipes) < 2:
             continue
         mine = [ff.PulseSequence(c, n, dt) for c, n, dt in recipes]
-        theirs = [ref.PulseSequence(c, n, dt) for c, n, dt in recipes]
-        for _ in range(4):      # same library, several sequences (plan reuse, other first occurrences)
+        for seq in range(4):    # same library, several sequences (plan reuse, other first occurrences)
             idx = rng.integers(0, len(recipes), int(rng.integers(2, 25)))
-            got = outcome(ff, ff.pulse_sequence.concatenate_without_filter_function,
-                          [mine[i] for i in idx])
-            want = outcome(ref, ref.pulse_sequence.concatenate_without_filter_function,
-                           [theirs[i] for i in idx])
+            got = outcome(ff.pulse_sequence.concatenate_without_filter_function, [mine[i] for i in idx])
+            want = ref(f'{nasty}/{lib}/{seq}', lambda m: joined(m, recipes, idx))
             assert len(got) == len(want)
             if len(got) == 2:
                 assert got == want
