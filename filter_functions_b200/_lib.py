@@ -76,6 +76,7 @@ EXPORTED_SYMBOLS = {
     'ffb_host_free': (c_int, [c_void_p, c_void_p]),
     'ffb_kernel_timing_enable': (c_int, [c_void_p, c_int]),
     'ffb_kernel_timing_read': (c_int, [c_void_p, _dp, POINTER(c_int64), c_int]),
+    'ffb_dispatch_log': (c_int, [c_void_p, c_void_p, c_int]),
     'ffb_shadow_enable_next': (c_int, [c_void_p, c_int]),
     'ffb_shadow_upload': (c_int, [c_void_p, c_void_p, c_size_t]),
     'ffb_shadow_query': (c_int, [c_void_p, c_void_p, c_size_t]),
@@ -266,6 +267,26 @@ def shadow_stats(ctx=None):
     n, nbytes, hits, hit_bytes = c_int(), c_size_t(), c_int64(), c_size_t()
     lib().ffb_shadow_stats(ctx, byref(n), byref(nbytes), byref(hits), byref(hit_bytes))
     return n.value, nbytes.value, hits.value, hit_bytes.value
+
+
+DISPATCH_LOG_MAX = 256
+
+
+class DispatchRecord(ctypes.Structure):
+    """``ffb_dispatch_record`` of include/ffb200.h."""
+    _fields_ = [('kernel', ctypes.c_char*64), ('prologue', ctypes.c_char*96)] + [
+        (name, c_int) for name in ('S', 'passes_per_chunk', 'n_pass', 'n_sp', 'pps', 'transposed', 'n_rb',
+                                   'n_wtiles', 'ctas_by_regs', 'block', 'n_blocks', 'n_omega')]
+
+
+def dispatch_log(ctx=None):
+    """What the control-matrix calls of a context launched since the last call, one dict per frequency
+    block, oldest first (``ffb_dispatch_log``); clears the record."""
+    ctx = context() if ctx is None else ctx
+    records = (DispatchRecord*DISPATCH_LOG_MAX)()
+    n = lib().ffb_dispatch_log(ctx, ctypes.addressof(records), DISPATCH_LOG_MAX)
+    return [{name: (getattr(rec, name).decode() if name in ('kernel', 'prologue') else getattr(rec, name))
+             for name, _ in DispatchRecord._fields_} for rec in records[:n]]
 
 
 def ptr(arr):

@@ -356,6 +356,18 @@ int ffb_kernel_timing_read(ffb_ctx* ctx, double* total_ms, int64_t* launches, in
   return FFB_OK;
 }
 
+int ffb_dispatch_log(ffb_ctx* ctx, ffb_dispatch_record* out, int capacity) {
+  if (!ctx) return FFB_EINVAL;
+  int n = 0;
+  if (out)
+    for (const auto& rec : ctx->dispatch_log) {
+      if (n >= capacity) break;
+      out[n++] = rec;
+    }
+  ctx->dispatch_log.clear();
+  return n;
+}
+
 // ------------------------------------------------------------------------------------------------
 // raw device memory
 // ------------------------------------------------------------------------------------------------

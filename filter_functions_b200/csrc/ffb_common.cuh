@@ -5,6 +5,7 @@
 
 #include <cstdint>
 #include <cstdio>
+#include <deque>
 #include <functional>
 #include <map>
 #include <string>
@@ -119,6 +120,9 @@ struct ffb_ctx {
   int64_t timed_launches = 0;
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> pending_events;
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> event_pool;
+
+  // what the control-matrix calls launched, per frequency block (ffb_dispatch_log)
+  std::deque<ffb_dispatch_record> dispatch_log;
 };
 
 int ffb_fail(ffb_ctx* ctx, int code, const char* fmt, ...);

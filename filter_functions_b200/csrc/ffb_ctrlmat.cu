@@ -1570,8 +1570,9 @@ constexpr int STAGE_TARGET_BYTES = 32 * 1024;
 constexpr int STAGE_MAX_BYTES = 48 * 1024;
 
 template <int MT, int NW>
-int launch_main(ffb_ctx* ctx, MainParams p, int n_wtiles, int n_rb, int S) {
+int launch_main(ffb_ctx* ctx, MainParams p, int n_wtiles, int n_rb, int S, ffb_dispatch_record& disp) {
   auto kern = ctrlmat_main_kernel<MT, NW>;
+  snprintf(disp.kernel, sizeof disp.kernel, "ctrlmat_main_kernel<%d, %d>", MT, NW);
   const size_t smem = (size_t)2 * p.stage_doubles * sizeof(double);
   FFB_TRY(ffb_func_smem(ctx, kern, smem));
   dim3 grid(n_wtiles, n_rb, S);
@@ -1584,8 +1585,10 @@ int launch_main(ffb_ctx* ctx, MainParams p, int n_wtiles, int n_rb, int S) {
 }
 
 template <int MT, int NW, int NP, int NSP, bool SPLIT = false>
-int launch_static(ffb_ctx* ctx, MainParams p, int n_wtiles, int n_rb, int S) {
+int launch_static(ffb_ctx* ctx, MainParams p, int n_wtiles, int n_rb, int S, ffb_dispatch_record& disp) {
   auto kern = ctrlmat_static_kernel<MT, NW, NP, NSP, SPLIT>;
+  snprintf(disp.kernel, sizeof disp.kernel, "ctrlmat_static_kernel<%d, %d, %d, %d, %s>", MT, NW, NP, NSP,
+           SPLIT ? "true" : "false");
   const size_t smem = (size_t)2 * p.stage_doubles * sizeof(double) + 16;  // + two mbarriers
   FFB_TRY(ffb_func_smem(ctx, kern, smem));
   dim3 grid(n_wtiles, n_rb, S);
@@ -1641,7 +1644,8 @@ int ffbi_ctrlmat_i8_prepare(ffb_ctx* ctx, int G, int rows, int n_krows, const do
                             const double* Cbar, const double* eigvals, const double* dt,
                             const double* t, DevBuf& stream, DevBuf& scales);
 int ffbi_ctrlmat_i8_run(ffb_ctx* ctx, int G, const double* omega, int n_omega, const DevBuf& stream,
-                        const DevBuf& scales, DevBuf& partial, int* S_out);
+                        const DevBuf& scales, DevBuf& partial, int* S_out, int* stages_per_chunk,
+                        int* n_stages_out, int* n_tiles_out);
 
 int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int n_omega,
                         const double* eigvals, const double* eigvecs, const double* propagators,
@@ -1690,6 +1694,7 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
   if (const char* e = getenv("FFB_CTRLMAT_SPLIT_IDENTITY")) split_tensor = split_tensor && atoi(e) != 0;
   const int split_t = split_tensor ? n_nops * (n_basis - 1) : 0;
   DevBuf Bbar, Cbar, stream, partial, i8_scales;
+  std::string prologue;  // for the dispatch record
   if (!fused_prologue) {
     FFB_TRY(Bbar.alloc(ctx, (size_t)G * n_jrows * dd * 16));
     FFB_TRY(Cbar.alloc(ctx, (size_t)G * n_krows * dd * 16));
@@ -1710,6 +1715,7 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
     };
     if (d == 2) FFB_TRY(launch(dfma_prologue_kernel<2>));
     else FFB_TRY(launch(dfma_prologue_kernel<3>));
+    prologue = d == 2 ? "dfma_prologue_kernel<2>" : "dfma_prologue_kernel<3>";
     FFB_LAUNCHED(ctx);
   } else if (d >= 2 && d <= 4) {
     const long long n_threads = (long long)G * (n_nops + n_basis);
@@ -1723,6 +1729,7 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
     if (d == 2) args(transform_small_kernel<2>);
     else if (d == 3) args(transform_small_kernel<3>);
     else args(transform_small_kernel<4>);
+    prologue = "transform_small_kernel<" + std::to_string(d) + ">";
     FFB_LAUNCHED(ctx);
   } else {
     const size_t smem = (size_t)8 * dd * sizeof(double);
@@ -1733,6 +1740,7 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
                                                     propagators, n_opers, n_coeffs, basis,
                                                     Bbar.as<double>(), Cbar.as<double>());
     FFB_LAUNCHED(ctx);
+    prologue = "transform_kernel";
   }
   if (fused_prologue) {
     // records written by dfma_prologue_kernel
@@ -1743,10 +1751,12 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
                                                           Bbar.as<double>(), Cbar.as<double>(),
                                                           eigvals, dt, t, stream.as<double>());
     FFB_LAUNCHED(ctx);
+    prologue += "+assemble_dfma_kernel";
   } else if (use_i8) {
     // digit stream of the coefficients + per-segment constants (ffb_ctrlmat_i8.cu)
     FFB_TRY(ffbi_ctrlmat_i8_prepare(ctx, G, rows, n_krows, Bbar.as<double>(), Cbar.as<double>(), eigvals,
                                     dt, t, stream, i8_scales));
+    prologue += "+i8_rowmax_kernel+i8_coeff_kernel";
   } else {
     // operators of a pass's segments in shared memory when they fit
     const size_t stage_bytes = (size_t)(geo.transposed ? 1 : 4) * (n_jrows + n_krows) * 2 * dd * sizeof(double);
@@ -1756,20 +1766,25 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
       assemble_kernel<true><<<blocks, 256, stage_bytes, ctx->stream>>>(
           geo, G, d, rows, n_jrows, n_krows, split_t, Bbar.as<double>(), Cbar.as<double>(), eigvals, dt, t,
           stream.as<double>());
+      prologue += "+assemble_kernel<true>";
     } else {
       assemble_kernel<false><<<blocks, 256, 0, ctx->stream>>>(
           geo, G, d, rows, n_jrows, n_krows, split_t, Bbar.as<double>(), Cbar.as<double>(), eigvals, dt, t,
           stream.as<double>());
+      prologue += "+assemble_kernel<false>";
     }
     FFB_LAUNCHED(ctx);
   }
 
   // ---- omega-dependent part, per block of frequencies (one block unless the caller asked for more)
   const size_t ld_out = (size_t)n_omega_all;
-  auto run_block = [&](const double* omega, int n_omega, double* out) -> int {
+  auto run_block = [&](const double* omega, int n_omega, double* out, ffb_dispatch_record& disp) -> int {
   if (use_i8) {
     int S_i8 = 1;
-    FFB_TRY(ffbi_ctrlmat_i8_run(ctx, G, omega, n_omega, stream, i8_scales, partial, &S_i8));
+    FFB_TRY(ffbi_ctrlmat_i8_run(ctx, G, omega, n_omega, stream, i8_scales, partial, &S_i8,
+                                &disp.passes_per_chunk, &disp.n_pass, &disp.n_wtiles));
+    snprintf(disp.kernel, sizeof disp.kernel, "ctrlmat_i8_kernel");
+    disp.S = S_i8;
     const size_t total = (size_t)n_nops * n_basis * n_omega;
     const unsigned fblocks = (unsigned)std::min<size_t>(ceil_div_sz(total, 256), (size_t)ctx->sm_count * 16);
     finalize_kernel<<<fblocks, 256, 0, ctx->stream>>>(S_i8, 96, n_nops, n_basis, 1, 1, n_omega, ld_out, 0,
@@ -1844,11 +1859,16 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
     int slot = -1;
     FFB_TRY(ffb_time_begin(ctx, &slot));
     const TrigConsts tc = trig_consts();
-#define FFB_DFMA_LAUNCH(R_, RF_, NP_) \
-  ctrlmat_dfma_kernel<R_, RF_, NP_><<<grid, DFMA_WARPS * 32, smem, ctx->stream>>>(q, tc)
+#define FFB_DFMA_LAUNCH(R_, RF_, NP_)                                                             \
+  ctrlmat_dfma_kernel<R_, RF_, NP_><<<grid, DFMA_WARPS * 32, smem, ctx->stream>>>(q, tc);        \
+  snprintf(disp.kernel, sizeof disp.kernel, "ctrlmat_dfma_kernel<%d, %d, %d>", R_, RF_, NP_)
     FFB_DFMA_DISPATCH(FFB_DFMA_LAUNCH)
     FFB_LAUNCHED(ctx);
     FFB_TRY(ffb_time_end(ctx, slot));
+    disp.S = S;
+    disp.passes_per_chunk = chunk;
+    disp.n_pass = G;
+    disp.n_wtiles = n_wt;
     const size_t total_out = (size_t)n_nops * n_basis * n_omega;
     const unsigned fblocks = (unsigned)std::min<size_t>(ceil_div_sz(total_out, 256), (size_t)ctx->sm_count * 16);
     finalize_kernel<<<fblocks, 256, 0, ctx->stream>>>(S, R, n_nops, n_basis, parts_j, parts_k, n_omega,
@@ -1952,37 +1972,40 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
   bool use_static8 = geo.n_pairs == 28 && !geo.transposed && p.pps == 1 &&
                      ((MT == 12 && p.n_sp >= 5 && p.n_sp <= 7) || (MT == 8 && p.n_sp >= 4 && p.n_sp <= 6));
   if (const char* e = getenv("FFB_CTRLMAT_STATIC")) use_static8 = use_static8 && atoi(e) != 0;
-  if (getenv("FFB_TRACE") && geo.n_pairs == 28)
-    fprintf(stderr, "[ffb trace] control matrix d = 8: MT %d n_sp %d pps %d transposed %d -> %s kernel\n", MT,
-            p.n_sp, p.pps, geo.transposed, use_static8 ? "static" : "generic");
   // d = 16 in the transposed layout (short pulses: the gate pulses and the joined pulse of config 5): 30 units
   // of four level pairs each + the diagonal unit per segment
   bool use_static16 = geo.n_pairs == 30 && geo.transposed && p.pps == 1 && MT == 12 && p.n_sp == 7;
   if (const char* e = getenv("FFB_CTRLMAT_STATIC")) use_static16 = use_static16 && atoi(e) != 0;
-  if (getenv("FFB_TRACE") && geo.n_pairs == 30)
-    fprintf(stderr, "[ffb trace] control matrix d = 16: MT %d n_sp %d pps %d transposed %d -> %s kernel\n", MT,
-            p.n_sp, p.pps, geo.transposed, use_static16 ? "static" : "generic");
+  disp.S = S;
+  disp.passes_per_chunk = ppc;
+  disp.n_pass = geo.n_pass;
+  disp.n_sp = p.n_sp;
+  disp.pps = p.pps;
+  disp.transposed = geo.transposed;
+  disp.n_rb = geo.n_rb;
+  disp.n_wtiles = n_wtiles;
+  disp.ctas_by_regs = ctas_by_regs;
   if (use_static16) {
-    FFB_TRY((launch_static<12, 4, 30, 7>(ctx, p, n_wtiles, geo.n_rb, S)));
+    FFB_TRY((launch_static<12, 4, 30, 7>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
   } else if (use_static8) {
-    if (MT == 12 && p.n_sp == 5) FFB_TRY((launch_static<12, 4, 28, 5>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else if (MT == 12 && p.n_sp == 6) FFB_TRY((launch_static<12, 4, 28, 6>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else if (MT == 12) FFB_TRY((launch_static<12, 4, 28, 7>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else if (p.n_sp == 4) FFB_TRY((launch_static<8, 4, 28, 4>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else if (p.n_sp == 5) FFB_TRY((launch_static<8, 4, 28, 5>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else FFB_TRY((launch_static<8, 4, 28, 6>(ctx, p, n_wtiles, geo.n_rb, S)));
+    if (MT == 12 && p.n_sp == 5) FFB_TRY((launch_static<12, 4, 28, 5>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else if (MT == 12 && p.n_sp == 6) FFB_TRY((launch_static<12, 4, 28, 6>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else if (MT == 12) FFB_TRY((launch_static<12, 4, 28, 7>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else if (p.n_sp == 4) FFB_TRY((launch_static<8, 4, 28, 4>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else if (p.n_sp == 5) FFB_TRY((launch_static<8, 4, 28, 5>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else FFB_TRY((launch_static<8, 4, 28, 6>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
   } else if (use_static) {
-    if (MT == 12 && p.n_sp == 2 && split_t) FFB_TRY((launch_static<12, 4, 6, 2, true>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else if (MT == 12 && p.n_sp == 2) FFB_TRY((launch_static<12, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else if (MT == 12) FFB_TRY((launch_static<12, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else if (MT == 10 && p.n_sp == 2) FFB_TRY((launch_static<10, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else if (MT == 10) FFB_TRY((launch_static<10, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else if (MT == 8 && p.n_sp == 2) FFB_TRY((launch_static<8, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else if (MT == 8) FFB_TRY((launch_static<8, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else if (p.n_sp == 2) FFB_TRY((launch_static<6, 8, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S)));
-    else FFB_TRY((launch_static<6, 8, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S)));
+    if (MT == 12 && p.n_sp == 2 && split_t) FFB_TRY((launch_static<12, 4, 6, 2, true>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else if (MT == 12 && p.n_sp == 2) FFB_TRY((launch_static<12, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else if (MT == 12) FFB_TRY((launch_static<12, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else if (MT == 10 && p.n_sp == 2) FFB_TRY((launch_static<10, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else if (MT == 10) FFB_TRY((launch_static<10, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else if (MT == 8 && p.n_sp == 2) FFB_TRY((launch_static<8, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else if (MT == 8) FFB_TRY((launch_static<8, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else if (p.n_sp == 2) FFB_TRY((launch_static<6, 8, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    else FFB_TRY((launch_static<6, 8, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
   } else {
-    FFB_DISPATCH_MT(MT, FFB_TRY((launch_main<MT_, NW_>(ctx, p, n_wtiles, geo.n_rb, S))));
+    FFB_DISPATCH_MT(MT, FFB_TRY((launch_main<MT_, NW_>(ctx, p, n_wtiles, geo.n_rb, S, disp))));
   }
 
   {
@@ -1998,9 +2021,24 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
   // block boundaries on multiples of 64 frequencies (the frequency tiles of all kernel variants)
   const int n_blocks = blocks ? std::max(1, std::min(blocks->n_blocks, ceil_div(n_omega_all, 64))) : 1;
   const int per_block = ceil_div(ceil_div(n_omega_all, n_blocks), 64) * 64;
+  const bool trace = getenv("FFB_TRACE") != nullptr;
   for (int w0 = 0; w0 < n_omega_all; w0 += per_block) {
     const int w1 = std::min(n_omega_all, w0 + per_block);
-    FFB_TRY(run_block(omega_all + w0, w1 - w0, out_all + 2 * (size_t)w0));
+    ffb_dispatch_record disp = {};
+    snprintf(disp.prologue, sizeof disp.prologue, "%s", prologue.c_str());
+    disp.block = w0 / per_block;
+    disp.n_blocks = ceil_div(n_omega_all, per_block);
+    disp.n_omega = w1 - w0;
+    FFB_TRY(run_block(omega_all + w0, w1 - w0, out_all + 2 * (size_t)w0, disp));
+    if (ctx->dispatch_log.size() >= FFB_DISPATCH_LOG_MAX) ctx->dispatch_log.pop_front();
+    ctx->dispatch_log.push_back(disp);
+    if (trace)
+      fprintf(stderr,
+              "[ffb trace] control matrix G %d d %d rows %d, block %d/%d (%d frequencies): %s after %s; S %d "
+              "passes_per_chunk %d n_pass %d n_sp %d pps %d transposed %d n_rb %d n_wtiles %d ctas_by_regs %d\n",
+              G, d, rows, disp.block + 1, disp.n_blocks, disp.n_omega, disp.kernel, disp.prologue, disp.S,
+              disp.passes_per_chunk, disp.n_pass, disp.n_sp, disp.pps, disp.transposed, disp.n_rb, disp.n_wtiles,
+              disp.ctas_by_regs);
     if (blocks && blocks->after_block) FFB_TRY(blocks->after_block(w0, w1));
   }
   return FFB_OK;

@@ -660,9 +660,11 @@ int ffbi_ctrlmat_i8_prepare(ffb_ctx* ctx, int G, int rows, int n_krows, const do
   return FFB_OK;
 }
 
-// Partial sums [S][96][n_omega] complex for one block of frequencies; *S_out chunks of the segment axis.
+// Partial sums [S][96][n_omega] complex for one block of frequencies; *S_out chunks of the segment axis
+// of *stages_per_chunk stages each, *n_stages_out stages, *n_tiles_out frequency tiles.
 int ffbi_ctrlmat_i8_run(ffb_ctx* ctx, int G, const double* omega, int n_omega, const DevBuf& stream,
-                        const DevBuf& scales, DevBuf& partial, int* S_out) {
+                        const DevBuf& scales, DevBuf& partial, int* S_out, int* stages_per_chunk,
+                        int* n_stages_out, int* n_tiles_out) {
   const int n_stages = ceil_div(G, I8_SEGS);
   const int n_tiles = ceil_div(n_omega, I8_W);
   // split of the segment axis: whole waves of CTAs (one CTA per SM), chunks short enough for int32
@@ -701,5 +703,8 @@ int ffbi_ctrlmat_i8_run(ffb_ctx* ctx, int G, const double* omega, int n_omega, c
   FFB_LAUNCHED(ctx);
   FFB_TRY(ffb_time_end(ctx, slot));
   *S_out = S;
+  *stages_per_chunk = spc;
+  *n_stages_out = n_stages;
+  *n_tiles_out = n_tiles;
   return FFB_OK;
 }

@@ -342,6 +342,32 @@ int ffb_shadow_stats(ffb_ctx* ctx, int* count, size_t* bytes, int64_t* hits, siz
 int ffb_kernel_timing_enable(ffb_ctx* ctx, int enable);
 int ffb_kernel_timing_read(ffb_ctx* ctx, double* total_ms, int64_t* launches, int reset);
 
+/* Record of the control-matrix dispatch: every control-matrix computation of a context (any entry point
+ * that computes one from scratch) appends one record per block of frequencies, naming the kernel
+ * instance it launched and the quantities that chose it.  Names are spelled as the demangled symbol
+ * without namespace and argument list, e.g. "ctrlmat_static_kernel<12, 4, 6, 2, true>".  For the DFMA
+ * kernels a "pass" is one segment, for the int8 kernel one stage of four segments; fields that do not
+ * apply to a kernel family are 0.  ffb_dispatch_log copies up to `capacity` records, oldest first, to
+ * `out` (may be NULL), clears the log and returns the number copied.  The log holds the last
+ * FFB_DISPATCH_LOG_MAX records. */
+#define FFB_DISPATCH_LOG_MAX 256
+typedef struct {
+  char kernel[64];       /* the omega-dependent kernel */
+  char prologue[96];     /* the omega-independent kernels before it, joined by '+' */
+  int S;                 /* chunks of the segment axis (partials summed by finalize_kernel) */
+  int passes_per_chunk;  /* passes per chunk (DFMA: segs_per_cta; int8: stages_per_chunk) */
+  int n_pass;
+  int n_sp;              /* pieces a pass is staged in */
+  int pps;               /* passes per stage */
+  int transposed;        /* level pairs of one segment in the K slots */
+  int n_rb;              /* row blocks */
+  int n_wtiles;          /* frequency tiles of the block */
+  int ctas_by_regs;      /* resident CTAs per SM the registers allow (sets the stage budget) */
+  int block, n_blocks;   /* this frequency block and the number of blocks of the call */
+  int n_omega;           /* frequencies in this block */
+} ffb_dispatch_record;
+int ffb_dispatch_log(ffb_ctx* ctx, ffb_dispatch_record* out, int capacity);
+
 #ifdef __cplusplus
 }
 #endif
