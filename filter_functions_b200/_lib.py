@@ -77,6 +77,7 @@ EXPORTED_SYMBOLS = {
     'ffb_kernel_timing_enable': (c_int, [c_void_p, c_int]),
     'ffb_kernel_timing_read': (c_int, [c_void_p, _dp, POINTER(c_int64), c_int]),
     'ffb_dispatch_log': (c_int, [c_void_p, c_void_p, c_int]),
+    'ffb_diag_dispatch_log': (c_int, [c_void_p, c_void_p, c_int]),
     'ffb_shadow_enable_next': (c_int, [c_void_p, c_int]),
     'ffb_shadow_upload': (c_int, [c_void_p, c_void_p, c_size_t]),
     'ffb_shadow_query': (c_int, [c_void_p, c_void_p, c_size_t]),
@@ -282,9 +283,19 @@ class DispatchRecord(ctypes.Structure):
 def dispatch_log(ctx=None):
     """What the control-matrix calls of a context launched since the last call, one dict per frequency
     block, oldest first (``ffb_dispatch_log``); clears the record."""
+    return _read_log(lib().ffb_dispatch_log, ctx)
+
+
+def diag_dispatch_log(ctx=None):
+    """What the diagonalisations of a context launched since the last call, one dict per call, oldest
+    first (``ffb_diag_dispatch_log``); clears the record."""
+    return _read_log(lib().ffb_diag_dispatch_log, ctx)
+
+
+def _read_log(fn, ctx):
     ctx = context() if ctx is None else ctx
     records = (DispatchRecord*DISPATCH_LOG_MAX)()
-    n = lib().ffb_dispatch_log(ctx, ctypes.addressof(records), DISPATCH_LOG_MAX)
+    n = fn(ctx, ctypes.addressof(records), DISPATCH_LOG_MAX)
     return [{name: (getattr(rec, name).decode() if name in ('kernel', 'prologue') else getattr(rec, name))
              for name, _ in DispatchRecord._fields_} for rec in records[:n]]
 

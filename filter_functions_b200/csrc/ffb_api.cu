@@ -356,16 +356,27 @@ int ffb_kernel_timing_read(ffb_ctx* ctx, double* total_ms, int64_t* launches, in
   return FFB_OK;
 }
 
-int ffb_dispatch_log(ffb_ctx* ctx, ffb_dispatch_record* out, int capacity) {
-  if (!ctx) return FFB_EINVAL;
+namespace {
+int copy_log(std::deque<ffb_dispatch_record>& log, ffb_dispatch_record* out, int capacity) {
   int n = 0;
   if (out)
-    for (const auto& rec : ctx->dispatch_log) {
+    for (const auto& rec : log) {
       if (n >= capacity) break;
       out[n++] = rec;
     }
-  ctx->dispatch_log.clear();
+  log.clear();
   return n;
+}
+}  // namespace
+
+int ffb_dispatch_log(ffb_ctx* ctx, ffb_dispatch_record* out, int capacity) {
+  if (!ctx) return FFB_EINVAL;
+  return copy_log(ctx->dispatch_log, out, capacity);
+}
+
+int ffb_diag_dispatch_log(ffb_ctx* ctx, ffb_dispatch_record* out, int capacity) {
+  if (!ctx) return FFB_EINVAL;
+  return copy_log(ctx->diag_dispatch_log, out, capacity);
 }
 
 // ------------------------------------------------------------------------------------------------

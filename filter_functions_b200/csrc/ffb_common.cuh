@@ -123,6 +123,8 @@ struct ffb_ctx {
 
   // what the control-matrix calls launched, per frequency block (ffb_dispatch_log)
   std::deque<ffb_dispatch_record> dispatch_log;
+  // what each diagonalisation launched (ffb_diag_dispatch_log)
+  std::deque<ffb_dispatch_record> diag_dispatch_log;
 };
 
 int ffb_fail(ffb_ctx* ctx, int code, const char* fmt, ...);

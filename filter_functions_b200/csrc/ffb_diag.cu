@@ -71,6 +71,20 @@ diag_kernel(int G, int d, int n_cops, const double* __restrict__ c_opers,
   }
   __syncwarp();
 
+  // H <- 2^-e H with e the exponent of its largest entry. The iteration is equivariant under powers of two
+  // except for the squares in its convergence test, which underflow for max|H| below ~1e-160 (0 sweeps,
+  // the diagonal returned as the eigenvalues) and overflow above ~1e154 (reported as not converged).
+  // Scaling by a power of two is exact, so no bit changes for H in between; NaN / Inf stay unscaled.
+  double hmax = 0.0;
+  for (int e = lane; e < dd; e += 32) hmax = fmax(hmax, fmax(fabs(H[2 * e]), fabs(H[2 * e + 1])));
+  for (int o = 16; o > 0; o >>= 1) hmax = fmax(hmax, __shfl_xor_sync(0xffffffffu, hmax, o));
+  int scale_exp = 0;
+  if (hmax > 0.0 && isfinite(hmax)) {
+    frexp(hmax, &scale_exp);
+    for (int e = lane; e < 2 * dd; e += 32) H[e] = ldexp(H[e], -scale_exp);
+  }
+  __syncwarp();
+
   double norm2 = 0.0;
   for (int e = lane; e < dd; e += 32) {
     const cplx h = lds_c(H, e);
@@ -163,7 +177,7 @@ diag_kernel(int G, int d, int n_cops, const double* __restrict__ c_opers,
 
   // ---- ascending order (stable), as numpy.linalg.eigh returns them
   if (lane < d) {
-    ev[lane] = H[2 * (lane * d + lane)];
+    ev[lane] = ldexp(H[2 * (lane * d + lane)], scale_exp);
     perm[lane] = lane;  // stays a valid permutation entry even if NaN eigenvalues make ranks collide
   }
   __syncwarp();
@@ -250,6 +264,21 @@ __device__ __forceinline__ void diag_small_one(int G, int g, int n_cops,
 #pragma unroll
     for (int c = r + 1; c < D; ++c) H[r][c] = cconj(H[c][r]);
   }
+  // H <- 2^-e H, e the exponent of its largest entry (exact; see diag_kernel)
+  double hmax = 0.0;
+#pragma unroll
+  for (int r = 0; r < D; ++r)
+#pragma unroll
+    for (int c = 0; c < D; ++c) hmax = fmax(hmax, fmax(fabs(H[r][c].re), fabs(H[r][c].im)));
+  int scale_exp = 0;
+  if (hmax > 0.0 && isfinite(hmax)) {
+    frexp(hmax, &scale_exp);
+#pragma unroll
+    for (int r = 0; r < D; ++r)
+#pragma unroll
+      for (int c = 0; c < D; ++c)
+        H[r][c] = cplx{ldexp(H[r][c].re, -scale_exp), ldexp(H[r][c].im, -scale_exp)};
+  }
   double norm2 = 0.0;
 #pragma unroll
   for (int r = 0; r < D; ++r)
@@ -335,7 +364,7 @@ __device__ __forceinline__ void diag_small_one(int G, int g, int n_cops,
   double ev[D];
   int rank[D];
 #pragma unroll
-  for (int j = 0; j < D; ++j) ev[j] = H[j][j].re;
+  for (int j = 0; j < D; ++j) ev[j] = ldexp(H[j][j].re, scale_exp);
 #pragma unroll
   for (int j = 0; j < D; ++j) {
     int rk = 0;
@@ -682,12 +711,32 @@ scan_apply_small_kernel(int n, int shift, const double2* __restrict__ local,
   for (int e = 0; e < DD; ++e) out[(size_t)(g + shift) * DD + e] = r[e];
 }
 
+// the scan kernel instances a diagonalisation launched, each named once in order of first launch, and
+// the number of scan levels (the dispatch record's prologue and S)
+struct ScanTrace {
+  std::string kernels;
+  int levels = 0;
+  void add(const char* name) {
+    if (kernels.find(name) != std::string::npos) return;
+    if (!kernels.empty()) kernels += '+';
+    kernels += name;
+  }
+  template <int D, int NT>
+  void add(const char* kernel) {
+    char name[64];
+    snprintf(name, sizeof name, "%s<%d, %d>", kernel, D, NT);
+    add(name);
+  }
+};
+
 // inclusive scan of n matrices `in` -> out[i + shift]; recursive over the block totals
 template <int D, int NT>
-int scan_small(ffb_ctx* ctx, int n, const double2* in, double2* out, int shift,
+int scan_small(ffb_ctx* ctx, ScanTrace& trace, int n, const double2* in, double2* out, int shift,
                const DiagArgs& da = DiagArgs{}) {
   constexpr int DD = D * D;
   const int nb = ceil_div(n, NT);
+  trace.levels++;
+  trace.add<D, NT>("scan_block_kernel");
   DevBuf local, totals, totals_incl;
   FFB_TRY(local.alloc(ctx, (size_t)n * DD * 16));
   FFB_TRY(totals.alloc(ctx, (size_t)nb * DD * 16));
@@ -697,6 +746,7 @@ int scan_small(ffb_ctx* ctx, int n, const double2* in, double2* out, int shift,
   kern<<<nb, NT, smem, ctx->stream>>>(n, in, local.as<double2>(), totals.as<double2>(), da);
   FFB_LAUNCHED(ctx);
   if (nb <= SCAN_PREFIX_MAX) {  // few blocks: their totals are combined inside the apply kernel
+    trace.add<D, NT>("scan_apply_prefix_kernel");
     scan_apply_prefix_kernel<D, NT><<<nb, NT, 0, ctx->stream>>>(
         n, shift, local.as<double2>(), totals.as<double2>(), out);
     FFB_LAUNCHED(ctx);
@@ -704,8 +754,9 @@ int scan_small(ffb_ctx* ctx, int n, const double2* in, double2* out, int shift,
   }
   if (nb > 1) {
     FFB_TRY(totals_incl.alloc(ctx, (size_t)nb * DD * 16));
-    FFB_TRY((scan_small<D, NT>(ctx, nb, totals.as<double2>(), totals_incl.as<double2>(), 0)));
+    FFB_TRY((scan_small<D, NT>(ctx, trace, nb, totals.as<double2>(), totals_incl.as<double2>(), 0)));
   }
+  trace.add<D, NT>("scan_apply_small_kernel");
   scan_apply_small_kernel<D, NT><<<ceil_div(n + 1, 256), 256, 0, ctx->stream>>>(
       n, shift, local.as<double2>(), nb > 1 ? totals_incl.as<double2>() : nullptr, out);
   FFB_LAUNCHED(ctx);
@@ -729,12 +780,28 @@ int ffbi_diagonalize(ffb_ctx* ctx, int G, int d, int n_cops, const double* c_ope
   FFB_TRY(ffb_conv_counter(ctx, &conv));
   static const bool small_ok = !(getenv("FFB_DIAG_SMALL") && atoi(getenv("FFB_DIAG_SMALL")) == 0);
   static const bool fuse_ok = !(getenv("FFB_DIAG_FUSED") && atoi(getenv("FFB_DIAG_FUSED")) == 0);
+  ffb_dispatch_record disp = {};
+  disp.n_pass = G;
+  ScanTrace trace;
+  auto logged = [&](int rc, int per_chunk) -> int {
+    if (rc != FFB_OK) return rc;
+    snprintf(disp.prologue, sizeof disp.prologue, "%s", trace.kernels.c_str());
+    disp.S = trace.levels;
+    disp.passes_per_chunk = per_chunk;
+    if (ctx->diag_dispatch_log.size() >= FFB_DISPATCH_LOG_MAX) ctx->diag_dispatch_log.pop_front();
+    ctx->diag_dispatch_log.push_back(disp);
+    return FFB_OK;
+  };
   if (d >= 2 && d <= 4 && small_ok && fuse_ok) {
     // diagonalisation fused into the block scan: thread per segment, propagator scanned from registers
     const DiagArgs da{n_cops, c_opers, c_coeffs, dt, eigvals, eigvecs, conv};
-    if (d == 2) return scan_small<2, 256>(ctx, G, nullptr, (double2*)propagators, 1, da);
-    if (d == 3) return scan_small<3, 128>(ctx, G, nullptr, (double2*)propagators, 1, da);
-    return scan_small<4, 128>(ctx, G, nullptr, (double2*)propagators, 1, da);
+    if (d == 2) {
+      snprintf(disp.kernel, sizeof disp.kernel, "scan_block_kernel<2, 256>");
+      return logged(scan_small<2, 256>(ctx, trace, G, nullptr, (double2*)propagators, 1, da), 256);
+    }
+    snprintf(disp.kernel, sizeof disp.kernel, "scan_block_kernel<%d, 128>", d);
+    if (d == 3) return logged(scan_small<3, 128>(ctx, trace, G, nullptr, (double2*)propagators, 1, da), 128);
+    return logged(scan_small<4, 128>(ctx, trace, G, nullptr, (double2*)propagators, 1, da), 128);
   }
   DevBuf piecewise, local, totals, prefix;
   FFB_TRY(piecewise.alloc(ctx, (size_t)G * dd * 16));
@@ -742,6 +809,7 @@ int ffbi_diagonalize(ffb_ctx* ctx, int G, int d, int n_cops, const double* c_ope
   FFB_TRY(totals.alloc(ctx, (size_t)n_chunks * dd * 16));
   FFB_TRY(prefix.alloc(ctx, (size_t)n_chunks * dd * 16));
   if (d >= 2 && d <= 4 && small_ok) {
+    snprintf(disp.kernel, sizeof disp.kernel, "diag_small_kernel<%d>", d);
     const unsigned nb = (unsigned)ceil_div(G, 128);
     if (d == 2)
       diag_small_kernel<2><<<nb, 128, 0, ctx->stream>>>(G, n_cops, c_opers, c_coeffs, dt, eigvals, eigvecs,
@@ -754,6 +822,7 @@ int ffbi_diagonalize(ffb_ctx* ctx, int G, int d, int n_cops, const double* c_ope
                                                         piecewise.as<double>(), conv);
     FFB_LAUNCHED(ctx);
   } else {
+    snprintf(disp.kernel, sizeof disp.kernel, "diag_kernel");
     const size_t smem = (size_t)DIAG_WARPS * (4 * dd + 2 * d) * sizeof(double);
     FFB_CUDA(ctx, cudaFuncSetAttribute(diag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)smem));
@@ -763,9 +832,10 @@ int ffbi_diagonalize(ffb_ctx* ctx, int G, int d, int n_cops, const double* c_ope
     FFB_LAUNCHED(ctx);
   }
   // running product Q_{g+1} = P_g ... P_0
-  if (d == 2) return scan_small<2, 256>(ctx, G, piecewise.as<double2>(), (double2*)propagators, 1);
-  if (d == 3) return scan_small<3, 128>(ctx, G, piecewise.as<double2>(), (double2*)propagators, 1);
-  if (d == 4) return scan_small<4, 128>(ctx, G, piecewise.as<double2>(), (double2*)propagators, 1);
+  const double2* P = piecewise.as<double2>();
+  if (d == 2) return logged(scan_small<2, 256>(ctx, trace, G, P, (double2*)propagators, 1), 256);
+  if (d == 3) return logged(scan_small<3, 128>(ctx, trace, G, P, (double2*)propagators, 1), 128);
+  if (d == 4) return logged(scan_small<4, 128>(ctx, trace, G, P, (double2*)propagators, 1), 128);
   {
     const size_t smem = (size_t)DIAG_WARPS * 4 * dd * sizeof(double);
     FFB_CUDA(ctx, cudaFuncSetAttribute(scan_local_kernel,
@@ -786,5 +856,7 @@ int ffbi_diagonalize(ffb_ctx* ctx, int G, int d, int n_cops, const double* c_ope
         G, d, L, local.as<double>(), prefix.as<double>(), propagators);
     FFB_LAUNCHED(ctx);
   }
-  return FFB_OK;
+  trace.levels = 1;
+  trace.kernels = "scan_local_kernel+scan_totals_kernel+scan_apply_from_kernel";
+  return logged(FFB_OK, L);
 }

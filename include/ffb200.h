@@ -349,7 +349,14 @@ int ffb_kernel_timing_read(ffb_ctx* ctx, double* total_ms, int64_t* launches, in
  * kernels a "pass" is one segment, for the int8 kernel one stage of four segments; fields that do not
  * apply to a kernel family are 0.  ffb_dispatch_log copies up to `capacity` records, oldest first, to
  * `out` (may be NULL), clears the log and returns the number copied.  The log holds the last
- * FFB_DISPATCH_LOG_MAX records. */
+ * FFB_DISPATCH_LOG_MAX records.
+ * ffb_diag_dispatch_log does the same for a log of its own, with one record per diagonalisation
+ * (ffb_diagonalize and the pulse entry points that diagonalise): `kernel` is the diagonaliser instance
+ * ("scan_block_kernel<4, 128>" when the diagonalisation is fused into the block scan,
+ * "diag_small_kernel<4>", "diag_kernel"), `prologue` the scan kernel instances it launched, each once, in
+ * order of first launch, `n_pass` = G segments, `passes_per_chunk` the segments per scan block or chunk
+ * (NT, or L for the generic scan) and `S` the number of scan levels (the block scan runs once per level);
+ * the other fields are 0. */
 #define FFB_DISPATCH_LOG_MAX 256
 typedef struct {
   char kernel[64];       /* the omega-dependent kernel */
@@ -367,6 +374,7 @@ typedef struct {
   int n_omega;           /* frequencies in this block */
 } ffb_dispatch_record;
 int ffb_dispatch_log(ffb_ctx* ctx, ffb_dispatch_record* out, int capacity);
+int ffb_diag_dispatch_log(ffb_ctx* ctx, ffb_dispatch_record* out, int capacity);
 
 #ifdef __cplusplus
 }
