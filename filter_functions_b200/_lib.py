@@ -46,6 +46,9 @@ EXPORTED_SYMBOLS = {
                                     + [c_int, c_void_p]),
     'ffb_infidelity': (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p,
                                c_int, c_int, c_void_p, c_int, c_void_p]),
+    'ffb_infidelity_derivative': (c_int, [c_void_p] + [c_int]*6 + [c_void_p]*12
+                                  + [c_int, c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p,
+                                     c_int, c_void_p]),
     'ffb_decay_amplitudes': (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int,
                                      c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     'ffb_dev_decay_amplitudes': (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int,

@@ -1099,6 +1099,97 @@ int ffb_infidelity(ffb_ctx* ctx, int n_lead, int n_nops, int n_sel, const int* i
   return ffbi_comm_check_error(ctx);
 }
 
+int ffb_infidelity_derivative(ffb_ctx* ctx, int G, int d, int n_cops, int n_nops, int n_basis,
+                              int n_omega, const double* c_opers, const double* c_coeffs,
+                              const double* eigvals, const double* eigvecs,
+                              const double* propagators, const double* omega, const double* basis,
+                              const double* n_opers, const double* n_coeffs, const double* dt,
+                              const double* t, const double* control_matrix, int n_ctrl,
+                              const int* ctrl_idx, int n_sel, const int* sel_idx,
+                              const double* spectrum, int spectrum_ndim,
+                              const double* n_coeffs_deps, int norm_d, double* out) {
+  FFB_TRY(enter(ctx));
+  const bool diag = !eigvals;
+  FFB_REQUIRE(ctx, c_opers && omega && basis && n_opers && n_coeffs && dt && t && ctrl_idx && sel_idx &&
+                       spectrum && out && (diag ? c_coeffs && !eigvecs && !propagators
+                                                : eigvecs && propagators),
+              "infidelity derivative: null pointer");
+  FFB_REQUIRE(ctx, d >= 1 && d <= 8,
+              "infidelity derivative: Hilbert-space dimension d = %d exceeds the supported maximum of 8 "
+              "of filter_functions_b200 (README: limits)", d);
+  FFB_REQUIRE(ctx, G >= 1 && n_cops >= 1 && n_nops >= 1 && n_basis >= 1 && n_omega >= 1 && n_ctrl >= 1 &&
+                       n_sel >= 1 && norm_d >= 1,
+              "infidelity derivative: bad shape");
+  FFB_REQUIRE(ctx, spectrum_ndim == 1 || spectrum_ndim == 2, "infidelity derivative: spectrum_ndim=%d",
+              spectrum_ndim);
+  for (int i = 0; i < n_ctrl; ++i)
+    FFB_REQUIRE(ctx, ctrl_idx[i] >= 0 && ctrl_idx[i] < n_cops,
+                "infidelity derivative: ctrl_idx[%d]=%d out of range", i, ctrl_idx[i]);
+  for (int i = 0; i < n_sel; ++i)
+    FFB_REQUIRE(ctx, sel_idx[i] >= 0 && sel_idx[i] < n_nops,
+                "infidelity derivative: sel_idx[%d]=%d out of range", i, sel_idx[i]);
+  const size_t dd = (size_t)d * d;
+  // one packed upload; arrays the pulse keeps mirrored on the device (its cached eigensystem and
+  // control matrix) are read from there
+  PackedUpload in(ctx);
+  const int i_co = in.add(c_opers, (size_t)n_cops * dd * 16);
+  const int i_cc = diag ? in.add(c_coeffs, (size_t)n_cops * G * 8) : -1;
+  const int i_ev = diag ? -1 : in.add(eigvals, (size_t)G * d * 8);
+  const int i_V = diag ? -1 : in.add(eigvecs, (size_t)G * dd * 16);
+  const int i_Q = diag ? -1 : in.add(propagators, (size_t)G * dd * 16);
+  const int i_om = in.add(omega, (size_t)n_omega * 8);
+  const int i_bs = in.add(basis, (size_t)n_basis * dd * 16);
+  const int i_no = in.add(n_opers, (size_t)n_nops * dd * 16);
+  const int i_nc = in.add(n_coeffs, (size_t)n_nops * G * 8);
+  const int i_dt = in.add(dt, (size_t)G * 8);
+  const int i_ts = in.add(t, (size_t)(G + 1) * 8);
+  const int i_B = control_matrix ? in.add(control_matrix, (size_t)n_nops * n_basis * n_omega * 16) : -1;
+  const int i_ci = in.add(ctrl_idx, (size_t)n_ctrl * sizeof(int));
+  const int i_si = in.add(sel_idx, (size_t)n_sel * sizeof(int));
+  const int i_sp = in.add(spectrum, (size_t)(spectrum_ndim == 2 ? n_sel : 1) * n_omega * 8);
+  const int i_dp = n_coeffs_deps ? in.add(n_coeffs_deps, (size_t)n_nops * n_ctrl * G * 8) : -1;
+  FFB_TRY(in.upload(ctx));
+  DevBuf ev, V, Q, B, res;
+  const double *ev_d, *V_d, *Q_d;
+  if (diag) {
+    FFB_TRY(ev.alloc(ctx, (size_t)G * d * 8));
+    FFB_TRY(V.alloc(ctx, (size_t)G * dd * 16));
+    FFB_TRY(Q.alloc(ctx, (size_t)(G + 1) * dd * 16));
+    FFB_TRY(ffbi_diagonalize(ctx, G, d, n_cops, in.d(i_co), in.d(i_cc), in.d(i_dt), ev.as<double>(),
+                             V.as<double>(), Q.as<double>()));
+    ev_d = ev.as<double>();
+    V_d = V.as<double>();
+    Q_d = Q.as<double>();
+  } else {
+    ev_d = in.d(i_ev);
+    V_d = in.d(i_V);
+    Q_d = in.d(i_Q);
+  }
+  const double* B_d;
+  if (control_matrix) {
+    B_d = in.d(i_B);
+  } else {
+    const int herm = (all_hermitian(n_opers, n_nops, d) ? FFB_HERM_NOPERS : 0) |
+                     basis_flags(basis, n_basis, d);
+    FFB_TRY(B.alloc(ctx, (size_t)n_nops * n_basis * n_omega * 16));
+    FFB_TRY(ffbi_control_matrix(ctx, G, d, n_nops, n_basis, n_omega, ev_d, V_d, Q_d, in.d(i_om),
+                                in.d(i_bs), in.d(i_no), in.d(i_nc), in.d(i_dt), in.d(i_ts), herm,
+                                B.as<double>()));
+    B_d = B.as<double>();
+  }
+  const size_t n_out = (size_t)n_sel * G * n_ctrl;
+  FFB_TRY(res.alloc(ctx, n_out * 8));
+  FFB_TRY(ffbi_infidelity_derivative(
+      ctx, G, d, n_nops, n_basis, n_omega, ev_d, V_d, Q_d, in.d(i_om), in.d(i_bs), in.d(i_no),
+      in.d(i_nc), in.d(i_dt), in.d(i_ts), in.d(i_co), B_d, n_ctrl,
+      reinterpret_cast<const int*>(in.d(i_ci)), n_sel, reinterpret_cast<const int*>(in.d(i_si)),
+      in.d(i_sp), spectrum_ndim, n_coeffs_deps ? in.d(i_dp) : nullptr, norm_d, res.as<double>()));
+  FFB_TRY(ffb_d2h(ctx, out, res.p, n_out * 8));
+  if (diag) FFB_TRY(ffb_conv_fetch(ctx));
+  FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return diag ? ffb_conv_check(ctx) : FFB_OK;
+}
+
 int ffb_decay_amplitudes(ffb_ctx* ctx, int P, int n_nops, int n_sel, const int* idx, int n_basis,
                          int n_omega, const double* B, const double* spectrum, int spectrum_ndim,
                          int spectrum_is_complex, const double* omega, double* out) {

@@ -275,6 +275,14 @@ int ffbi_control_matrix_intermediates(ffb_ctx* ctx, int G, int d, int n_nops, in
                                       double* eigvecs_propagated, double* basis_transformed,
                                       double* phase_factors, double* first_order_integral,
                                       double* step, double* cumulative);
+int ffbi_infidelity_derivative(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int n_omega,
+                               const double* eigvals, const double* eigvecs,
+                               const double* propagators, const double* omega, const double* basis,
+                               const double* n_opers, const double* n_coeffs, const double* dt,
+                               const double* t, const double* c_opers, const double* control_matrix,
+                               int n_ctrl, const int* ctrl_idx, int n_sel, const int* sel_idx,
+                               const double* spectrum, int spectrum_ndim,
+                               const double* n_coeffs_deps, int norm_d, double* out);
 int ffbi_control_matrix_periodic(ffb_ctx* ctx, int n_nops, int n_basis, int n_omega, int repeats,
                                  const double* phases, const double* B, const double* L,
                                  int l_is_complex, double* out);

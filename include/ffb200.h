@@ -112,6 +112,29 @@ int ffb_infidelity(ffb_ctx* ctx, int n_lead, int n_nops, int n_sel, const int* i
                    const double* F, const double* spectrum, int spectrum_ndim,
                    int spectrum_is_complex, const double* omega, int d, double* out);
 
+/* ---- gradient: derivative of the infidelity with respect to every control amplitude ----------------
+ * ff.infidelity_derivative (DESIGN.md section 4.11): out[a, g, h] = dI_a / du_h(g) of the first-order
+ * infidelity I_a = trapezoid(S_a F_aa) / (2 pi norm_d) of ffb_infidelity, for a traceless basis
+ * (F_aa = sum_k |B_ak|^2), with H_g = sum_i c_coeffs[i,g] c_opers[i].  Inputs as in
+ * ffb_control_matrix_from_scratch, plus
+ *   c_opers (n_cops,d,d) c128 | c_coeffs (n_cops,G) f64, only read when eigvals is NULL
+ *   eigvals, eigvecs, propagators: the pulse's diagonalisation, or all three NULL: diagonalised here
+ *   control_matrix (n_nops,n_basis,n_omega) c128 of all noise operators, or NULL: computed here
+ *   ctrl_idx (n_ctrl) rows of c_opers to differentiate by | sel_idx (n_sel) rows of n_opers
+ *   spectrum f64: spectrum_ndim 1: (n_omega) | 2: (n_sel,n_omega)
+ *   n_coeffs_deps (n_nops,n_ctrl,G) f64 d n_coeffs[a,g] / d c_coeffs[ctrl_idx[h],g], or NULL (zero)
+ *   out (n_sel,G,n_ctrl) f64.
+ * d <= 8.  Deterministic: the sums over frequencies and segments run in a fixed order. */
+int ffb_infidelity_derivative(ffb_ctx* ctx, int G, int d, int n_cops, int n_nops, int n_basis,
+                              int n_omega, const double* c_opers, const double* c_coeffs,
+                              const double* eigvals, const double* eigvecs,
+                              const double* propagators, const double* omega, const double* basis,
+                              const double* n_opers, const double* n_coeffs, const double* dt,
+                              const double* t, const double* control_matrix, int n_ctrl,
+                              const int* ctrl_idx, int n_sel, const int* sel_idx,
+                              const double* spectrum, int spectrum_ndim,
+                              const double* n_coeffs_deps, int norm_d, double* out);
+
 /* ---- f1 (SURVEY 8f rank 1): decay amplitudes ---------------------------------------------------
  * Replaces numeric.calculate_decay_amplitudes (numeric.py:1194-1337) with the integrand of
  * numeric._get_integrand for a control matrix (numeric.py:259-374, einsum '...ko,...o,...lo->...klo'):
