@@ -23,6 +23,11 @@ int ffb_fail(ffb_ctx* ctx, int code, const char* fmt, ...) {
   return code;
 }
 
+bool ffb_trace() {
+  static const bool on = getenv("FFB_TRACE") && atoi(getenv("FFB_TRACE")) != 0;
+  return on;
+}
+
 int ffb_pool_alloc(ffb_ctx* ctx, size_t bytes, void** ptr) {
   bytes = (bytes + 511) & ~(size_t)511;
   auto it = ctx->free_blocks.lower_bound(bytes);
@@ -578,22 +583,17 @@ bool first_is_identity(const double* basis, int d) {
   return true;
 }
 
-int basis_flags(const double* basis, int n_basis, int d) {
-  return (all_hermitian(basis, n_basis, d) ? FFB_HERM_BASIS : 0) |
+// Hermiticity and identity flags of the noise operators and the basis (FFB_HERM_*, FFB_BASIS_IDENTITY0)
+int herm_flags(const double* n_opers, int n_nops, const double* basis, int n_basis, int d) {
+  return (all_hermitian(n_opers, n_nops, d) ? FFB_HERM_NOPERS : 0) |
+         (all_hermitian(basis, n_basis, d) ? FFB_HERM_BASIS : 0) |
          (n_basis >= 1 && first_is_identity(basis, d) ? FFB_BASIS_IDENTITY0 : 0);
 }
 
-struct Upload {
-  DevBuf buf;
-  const void* shadow = nullptr;  // the host bytes are mirrored on the device already
-  int put(ffb_ctx* ctx, const void* host, size_t bytes) {
-    shadow = ffb_shadow_lookup(ctx, host, bytes);
-    if (shadow) return FFB_OK;
-    FFB_TRY(buf.alloc(ctx, bytes));
-    return ffb_h2d(ctx, buf.p, host, bytes);
-  }
-  const double* d() const { return shadow ? static_cast<const double*>(shadow) : buf.as<double>(); }
-};
+// elements of a spectrum of shape (n_omega,), (n_sel, n_omega) or (n_sel, n_sel, n_omega)
+size_t spectrum_elems(int ndim, int n_sel, int n_omega) {
+  return (ndim == 1 ? 1 : ndim == 2 ? (size_t)n_sel : (size_t)n_sel * n_sel) * n_omega;
+}
 
 int enter(ffb_ctx* ctx) {
   if (!ctx) return FFB_EINVAL;
@@ -601,72 +601,97 @@ int enter(ffb_ctx* ctx) {
   return FFB_OK;
 }
 
-// Several small host arrays -> ONE page-locked staging block -> ONE host-to-device copy.  A pageable
-// cudaMemcpyAsync costs ~10 us of driver time per call and blocks the host for the larger ones; a
-// pulse has 8-9 input arrays of 0.1-500 KB each.  The staging block belongs to the context and is
-// reused by the next call (every host-pointer entry point is synchronous on return).
+// All host inputs of one call -> ONE page-locked staging block -> as few host-to-device copies as the
+// sizes allow.  A pageable cudaMemcpyAsync costs ~10 us of driver time per call and blocks the host for
+// the larger ones; a pulse has 8-9 input arrays of 0.1-500 KB each.  The staging block belongs to the
+// context and is reused by the next call, so an entry point calls upload() exactly once: a second
+// upload() would overwrite staged bytes whose copy may still be in flight.  (Every host-pointer entry
+// point is synchronous on return, so the next call finds the block free.)
 struct PackedUpload {
   static constexpr size_t ALIGN = 256;
   static constexpr size_t PACK_LIMIT = (size_t)512 << 10;  // larger parts are copied from where they lie
   static constexpr size_t RUN_BYTES = (size_t)128 << 10;   // a run of packed parts is sent at this size
   std::vector<const void*> src, mirror;
   std::vector<size_t> bytes, offset;
-  size_t total = 0;
+  size_t packed = 0, large = 0;  // bytes through the staging block, bytes copied from where they lie
   DevBuf dev;
-  ffb_ctx* owner = nullptr;
-  explicit PackedUpload(ffb_ctx* ctx = nullptr) : owner(ctx) {}
+  ffb_ctx* ctx;
+  explicit PackedUpload(ffb_ctx* c) : ctx(c) {}
   int add(const void* host, size_t n) {
     // a part that is mirrored on the device already (a cached result array) is not sent again
-    const void* m = owner ? ffb_shadow_lookup(owner, host, n) : nullptr;
+    const void* m = ffb_shadow_lookup(ctx, host, n);
+    size_t& end = !m && n > PACK_LIMIT ? large : packed;
     src.push_back(host);
     mirror.push_back(m);
     bytes.push_back(m ? 0 : n);
-    offset.push_back(total);
-    if (!m) total += (n + ALIGN - 1) & ~(ALIGN - 1);
+    offset.push_back(end);
+    if (!m) end += (n + ALIGN - 1) & ~(ALIGN - 1);
     return (int)src.size() - 1;
   }
-  int upload(ffb_ctx* ctx) {
-    if (ctx->stage_bytes < total) {
+  // device layout: the staging block's layout, then the large parts
+  char* at(size_t i) const { return dev.as<char>() + offset[i] + (bytes[i] > PACK_LIMIT ? packed : 0); }
+  int upload() {
+    if (ctx->stage_bytes < packed) {
       if (ctx->stage_host) FFB_CUDA(ctx, cudaFreeHost(ctx->stage_host));
       ctx->stage_host = nullptr;
       ctx->stage_bytes = 0;
-      const size_t want = std::max<size_t>(2 * total, (size_t)1 << 20);
+      const size_t want = std::max<size_t>(2 * packed, (size_t)1 << 20);
       FFB_CUDA(ctx, cudaHostAlloc(&ctx->stage_host, want, cudaHostAllocDefault));
       ctx->stage_bytes = want;
     }
     char* stage = static_cast<char*>(ctx->stage_host);
-    char* d0 = nullptr;
-    FFB_TRY(dev.alloc(ctx, total ? total : 8));
-    d0 = static_cast<char*>(dev.p);
-    // the device block mirrors the staging layout: runs of consecutive small parts travel in one copy
-    // out of the staging block, a large part in its own copy straight from the caller's array (which
-    // is page-locked already when it is one of the library's result arrays)
+    FFB_TRY(dev.alloc(ctx, packed + large));
+    char* d0 = dev.as<char>();
+    // runs of consecutive small parts travel in one copy out of the staging block, a large part in its
+    // own copy straight from the caller's array (which is page-locked already when it is one of the
+    // library's result arrays)
     size_t run_begin = 0, run_end = 0;
     auto flush = [&]() -> int {
       if (run_end > run_begin) FFB_TRY(ffb_h2d(ctx, d0 + run_begin, stage + run_begin, run_end - run_begin));
+      run_begin = run_end = 0;
       return FFB_OK;
     };
     for (size_t i = 0; i < src.size(); ++i) {
       if (!bytes[i]) continue;
-      if (bytes[i] <= PACK_LIMIT) {
-        std::memcpy(stage + offset[i], src[i], bytes[i]);
-        if (run_end == run_begin) run_begin = offset[i];
-        run_end = offset[i] + bytes[i];
-        if (run_end - run_begin >= RUN_BYTES) {  // send what is packed while the rest is being packed
-          FFB_TRY(flush());
-          run_begin = run_end = 0;
-        }
-      } else {
-        FFB_TRY(flush());
-        run_begin = run_end = 0;
-        FFB_TRY(ffb_h2d(ctx, d0 + offset[i], src[i], bytes[i]));
+      if (bytes[i] > PACK_LIMIT) {
+        FFB_TRY(ffb_h2d(ctx, at(i), src[i], bytes[i]));
+        continue;
       }
+      std::memcpy(stage + offset[i], src[i], bytes[i]);
+      if (run_end == run_begin) run_begin = offset[i];
+      run_end = offset[i] + bytes[i];
+      if (run_end - run_begin >= RUN_BYTES) FFB_TRY(flush());  // send what is packed while the rest is packed
     }
     return flush();
   }
-  const double* d(int i) const {
-    if (mirror[i]) return static_cast<const double*>(mirror[i]);
-    return reinterpret_cast<const double*>(static_cast<const char*>(dev.p) + offset[i]);
+  template <typename T = double>
+  const T* d(int i) const {
+    return static_cast<const T*>(mirror[i] ? mirror[i] : static_cast<const void*>(at(i)));
+  }
+};
+
+// `to` waits for the work enqueued on `from` so far (through the context's copy event `ev`)
+int after(ffb_ctx* ctx, int ev, cudaStream_t from, cudaStream_t to) {
+  FFB_CUDA(ctx, cudaEventRecord(ctx->copy_ev[ev], from));
+  FFB_CUDA(ctx, cudaStreamWaitEvent(to, ctx->copy_ev[ev], 0));
+  return FFB_OK;
+}
+
+// enqueue on the copy stream the strided download of frequencies [w0, w1) of every row of a
+// (rows, n_omega) complex result
+int download_freqs(ffb_ctx* ctx, double* host, const double* dev, size_t rows, int n_omega, int w0, int w1) {
+  const size_t pitch = (size_t)n_omega * 16, off = (size_t)w0 * 16;
+  FFB_CUDA(ctx, cudaMemcpy2DAsync(reinterpret_cast<char*>(host) + off, pitch,
+                                  reinterpret_cast<const char*>(dev) + off, pitch, (size_t)(w1 - w0) * 16,
+                                  rows, cudaMemcpyDeviceToHost, ctx->copy_stream));
+  return FFB_OK;
+}
+
+// microseconds since construction, for the FFB_TRACE timelines
+struct TraceClock {
+  const std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
+  double operator()() const {
+    return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - t0).count();
   }
 };
 
@@ -857,16 +882,17 @@ int ffb_diagonalize(ffb_ctx* ctx, int G, int d, int n_cops, const double* c_oper
   FFB_CHECK_DIM(ctx, d);
   FFB_REQUIRE(ctx, G >= 1 && d >= 1 && d <= 32, "diagonalize: G=%d, d=%d unsupported", G, d);
   const size_t dd = (size_t)d * d;
-  Upload ops, coeffs, dts;
+  PackedUpload in(ctx);
   DevBuf ev, V, Q;
   const size_t n_mats = c_coeffs ? (size_t)n_cops : (size_t)G;
-  FFB_TRY(ops.put(ctx, c_opers, n_mats * dd * 16));
-  if (c_coeffs) FFB_TRY(coeffs.put(ctx, c_coeffs, (size_t)n_cops * G * 8));
-  FFB_TRY(dts.put(ctx, dt, (size_t)G * 8));
+  const int i_co = in.add(c_opers, n_mats * dd * 16);
+  const int i_cc = c_coeffs ? in.add(c_coeffs, (size_t)n_cops * G * 8) : -1;
+  const int i_dt = in.add(dt, (size_t)G * 8);
+  FFB_TRY(in.upload());
   FFB_TRY(ev.alloc(ctx, (size_t)G * d * 8));
   FFB_TRY(V.alloc(ctx, (size_t)G * dd * 16));
   FFB_TRY(Q.alloc(ctx, (size_t)(G + 1) * dd * 16));
-  FFB_TRY(ffbi_diagonalize(ctx, G, d, n_cops, ops.d(), c_coeffs ? coeffs.d() : nullptr, dts.d(),
+  FFB_TRY(ffbi_diagonalize(ctx, G, d, n_cops, in.d(i_co), c_coeffs ? in.d(i_cc) : nullptr, in.d(i_dt),
                            ev.as<double>(), V.as<double>(), Q.as<double>()));
   FFB_TRY(ffb_d2h(ctx, eigvals, ev.p, (size_t)G * d * 8));
   FFB_TRY(ffb_d2h(ctx, eigvecs, V.p, (size_t)G * dd * 16));
@@ -891,15 +917,10 @@ int ffb_control_matrix_from_scratch(ffb_ctx* ctx, int G, int d, int n_nops, int 
   const bool keep = ctx->shadow_next;
   ctx->shadow_next = false;
   const size_t dd = (size_t)d * d;
-  const int herm = (all_hermitian(n_opers, n_nops, d) ? FFB_HERM_NOPERS : 0) |
-                   basis_flags(basis, n_basis, d);
+  const int herm = herm_flags(n_opers, n_nops, basis, n_basis, d);
   FFB_TRY(ensure_copy_stream(ctx));
   ffb_shadow_drop_range(ctx, out, (size_t)n_nops * n_basis * n_omega * 16);
-  static const bool trace = getenv("FFB_TRACE") && atoi(getenv("FFB_TRACE")) != 0;
-  const auto t_enter = std::chrono::steady_clock::now();
-  auto since = [&]() {
-    return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - t_enter).count();
-  };
+  const TraceClock since;
   PackedUpload in(ctx);
   DevBuf B;
   CopyStreamDrain drain{ctx};
@@ -912,22 +933,15 @@ int ffb_control_matrix_from_scratch(ffb_ctx* ctx, int G, int d, int n_nops, int 
   const int i_nc = in.add(n_coeffs, (size_t)n_nops * G * 8);
   const int i_dt = in.add(dt, (size_t)G * 8);
   const int i_ts = in.add(t, (size_t)(G + 1) * 8);
-  FFB_TRY(in.upload(ctx));
+  FFB_TRY(in.upload());
   const size_t out_bytes = (size_t)n_nops * n_basis * n_omega * 16;
   FFB_TRY(B.alloc(ctx, out_bytes));
   // the rows of a finished block of frequencies are downloaded while the next block is computed
-  cudaStream_t cs = ctx->copy_stream;
-  const size_t pitch = (size_t)n_omega * 16;
   FreqBlocks fb;
   fb.n_blocks = pipeline_blocks(out_bytes, n_omega);
   fb.after_block = [&](int w0, int w1) -> int {
-    FFB_CUDA(ctx, cudaEventRecord(ctx->copy_ev[1], ctx->stream));
-    FFB_CUDA(ctx, cudaStreamWaitEvent(cs, ctx->copy_ev[1], 0));
-    FFB_CUDA(ctx, cudaMemcpy2DAsync(reinterpret_cast<char*>(out) + (size_t)w0 * 16, pitch,
-                                    static_cast<const char*>(B.p) + (size_t)w0 * 16, pitch,
-                                    (size_t)(w1 - w0) * 16, (size_t)n_nops * n_basis,
-                                    cudaMemcpyDeviceToHost, cs));
-    return FFB_OK;
+    FFB_TRY(after(ctx, 1, ctx->stream, ctx->copy_stream));
+    return download_freqs(ctx, out, B.as<double>(), (size_t)n_nops * n_basis, n_omega, w0, w1);
   };
   FFB_TRY(ffbi_control_matrix(ctx, G, d, n_nops, n_basis, n_omega, in.d(i_ev), in.d(i_V), in.d(i_Q),
                               in.d(i_om), in.d(i_bs), in.d(i_no), in.d(i_nc), in.d(i_dt), in.d(i_ts),
@@ -935,8 +949,8 @@ int ffb_control_matrix_from_scratch(ffb_ctx* ctx, int G, int d, int n_nops, int 
   const double us_enqueued = since();
   FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   const double us_main = since();
-  FFB_CUDA(ctx, cudaStreamSynchronize(cs));
-  if (trace)
+  FFB_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream));
+  if (ffb_trace())
     fprintf(stderr, "[ffb trace] control matrix: all work enqueued %.0f us, main stream done %.0f us, "
             "copy stream done %.0f us (%d blocks)\n", us_enqueued, us_main, since(), fb.n_blocks);
   if (keep) ffb_shadow_retain(ctx, B, out, out_bytes, {{0, out_bytes}});
@@ -963,17 +977,18 @@ int ffb_control_matrix_intermediates(ffb_ctx* ctx, int G, int d, int n_nops, int
   FFB_REQUIRE(ctx, G >= 1 && d >= 1 && d <= 32 && n_nops >= 1 && n_basis >= 1 && n_omega >= 1,
               "control matrix intermediates: bad shape");
   const size_t dd = (size_t)d * d;
-  Upload ev, V, Q, om, bs, no, nc, dts, ts;
+  PackedUpload in(ctx);
   DevBuf B, Bt, Up, Ct, Ph, In, St, Cu;
-  FFB_TRY(ev.put(ctx, eigvals, (size_t)G * d * 8));
-  FFB_TRY(V.put(ctx, eigvecs, (size_t)G * dd * 16));
-  FFB_TRY(Q.put(ctx, propagators, (size_t)G * dd * 16));
-  FFB_TRY(om.put(ctx, omega, (size_t)n_omega * 8));
-  FFB_TRY(bs.put(ctx, basis, (size_t)n_basis * dd * 16));
-  FFB_TRY(no.put(ctx, n_opers, (size_t)n_nops * dd * 16));
-  FFB_TRY(nc.put(ctx, n_coeffs, (size_t)n_nops * G * 8));
-  FFB_TRY(dts.put(ctx, dt, (size_t)G * 8));
-  FFB_TRY(ts.put(ctx, t, (size_t)(G + 1) * 8));
+  const int i_ev = in.add(eigvals, (size_t)G * d * 8);
+  const int i_V = in.add(eigvecs, (size_t)G * dd * 16);
+  const int i_Q = in.add(propagators, (size_t)G * dd * 16);
+  const int i_om = in.add(omega, (size_t)n_omega * 8);
+  const int i_bs = in.add(basis, (size_t)n_basis * dd * 16);
+  const int i_no = in.add(n_opers, (size_t)n_nops * dd * 16);
+  const int i_nc = in.add(n_coeffs, (size_t)n_nops * G * 8);
+  const int i_dt = in.add(dt, (size_t)G * 8);
+  const int i_ts = in.add(t, (size_t)(G + 1) * 8);
+  FFB_TRY(in.upload());
   const size_t per_step = (size_t)n_nops * n_basis * n_omega * 16;
   const size_t b_bt = (size_t)n_nops * G * dd * 16, b_up = (size_t)G * dd * 16,
                b_ct = (size_t)G * n_basis * dd * 16, b_ph = (size_t)G * n_omega * 16,
@@ -988,9 +1003,9 @@ int ffb_control_matrix_intermediates(ffb_ctx* ctx, int G, int d, int n_nops, int
   FFB_TRY(St.alloc(ctx, b_st));
   FFB_TRY(Cu.alloc(ctx, b_cu));
   FFB_TRY(ffbi_control_matrix_intermediates(
-      ctx, G, d, n_nops, n_basis, n_omega, ev.d(), V.d(), Q.d(), om.d(), bs.d(), no.d(), nc.d(),
-      dts.d(), ts.d(), B.as<double>(), Bt.as<double>(), Up.as<double>(), Ct.as<double>(),
-      Ph.as<double>(), In.as<double>(), St.as<double>(), Cu.as<double>()));
+      ctx, G, d, n_nops, n_basis, n_omega, in.d(i_ev), in.d(i_V), in.d(i_Q), in.d(i_om), in.d(i_bs),
+      in.d(i_no), in.d(i_nc), in.d(i_dt), in.d(i_ts), B.as<double>(), Bt.as<double>(), Up.as<double>(),
+      Ct.as<double>(), Ph.as<double>(), In.as<double>(), St.as<double>(), Cu.as<double>()));
   FFB_TRY(ffb_d2h(ctx, out, B.p, per_step));
   FFB_TRY(ffb_d2h(ctx, n_opers_transformed, Bt.p, b_bt));
   FFB_TRY(ffb_d2h(ctx, eigvecs_propagated, Up.p, b_up));
@@ -1009,13 +1024,14 @@ int ffb_filter_function(ffb_ctx* ctx, int P, int n_nops, int n_basis, int n_omeg
   FFB_REQUIRE(ctx, B && F, "filter function: null pointer");
   FFB_REQUIRE(ctx, P >= 1 && n_nops >= 1 && n_basis >= 1 && n_omega >= 1,
               "filter function: bad shape");
-  Upload Bd;
+  PackedUpload in(ctx);
   DevBuf Fd;
   const size_t L = (size_t)P * n_nops;
   const size_t f_bytes = L * L * (generalized ? (size_t)n_basis * n_basis : 1) * n_omega * 16;
-  FFB_TRY(Bd.put(ctx, B, L * n_basis * n_omega * 16));
+  const int i_B = in.add(B, L * n_basis * n_omega * 16);
+  FFB_TRY(in.upload());
   FFB_TRY(Fd.alloc(ctx, f_bytes));
-  FFB_TRY(ffbi_filter_function(ctx, P, n_nops, n_basis, n_omega, Bd.d(), generalized,
+  FFB_TRY(ffbi_filter_function(ctx, P, n_nops, n_basis, n_omega, in.d(i_B), generalized,
                                Fd.as<double>()));
   FFB_TRY(ffb_d2h(ctx, F, Fd.p, f_bytes));
   FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1030,18 +1046,18 @@ int ffb_control_matrix_from_atomic(ffb_ctx* ctx, int P, int n_nops, int n_basis,
   FFB_REQUIRE(ctx, B_atomic && out && (P == 1 || (phases && Q_liouville)),
               "from_atomic: null pointer");
   FFB_REQUIRE(ctx, P >= 1 && n_nops >= 1 && n_basis >= 1 && n_omega >= 1, "from_atomic: bad shape");
-  Upload ph, Ba, Q;
+  PackedUpload in(ctx);
   DevBuf O;
   const size_t pulse_bytes = (size_t)n_nops * n_basis * n_omega * 16;
-  if (P > 1) {
-    FFB_TRY(ph.put(ctx, phases, (size_t)(P - 1) * n_omega * 16));
-    FFB_TRY(Q.put(ctx, Q_liouville, (size_t)(P - 1) * n_basis * n_basis * (q_is_complex ? 16 : 8)));
-  }
-  FFB_TRY(Ba.put(ctx, B_atomic, P * pulse_bytes));
+  const int i_ph = P > 1 ? in.add(phases, (size_t)(P - 1) * n_omega * 16) : -1;
+  const int i_Q = P > 1 ? in.add(Q_liouville, (size_t)(P - 1) * n_basis * n_basis * (q_is_complex ? 16 : 8))
+                        : -1;
+  const int i_Ba = in.add(B_atomic, P * pulse_bytes);
+  FFB_TRY(in.upload());
   const size_t out_bytes = (correlations ? P : 1) * pulse_bytes;
   FFB_TRY(O.alloc(ctx, out_bytes));
-  FFB_TRY(ffbi_from_atomic(ctx, P, n_nops, n_basis, n_omega, P > 1 ? ph.d() : nullptr, Ba.d(),
-                           P > 1 ? Q.d() : nullptr, q_is_complex, correlations, O.as<double>()));
+  FFB_TRY(ffbi_from_atomic(ctx, P, n_nops, n_basis, n_omega, P > 1 ? in.d(i_ph) : nullptr, in.d(i_Ba),
+                           P > 1 ? in.d(i_Q) : nullptr, q_is_complex, correlations, O.as<double>()));
   FFB_TRY(ffb_d2h(ctx, out, O.p, out_bytes));
   FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return FFB_OK;
@@ -1054,15 +1070,16 @@ int ffb_control_matrix_periodic(ffb_ctx* ctx, int n_nops, int n_basis, int n_ome
   FFB_REQUIRE(ctx, phases && B && L && out, "periodic control matrix: null pointer");
   FFB_REQUIRE(ctx, n_nops >= 1 && n_basis >= 1 && n_omega >= 1 && repeats >= 1,
               "periodic control matrix: bad shape");
-  Upload ph, Bd, Ld;
+  PackedUpload in(ctx);
   DevBuf O;
   const size_t b_bytes = (size_t)n_nops * n_basis * n_omega * 16;
-  FFB_TRY(ph.put(ctx, phases, (size_t)n_omega * 16));
-  FFB_TRY(Bd.put(ctx, B, b_bytes));
-  FFB_TRY(Ld.put(ctx, L, (size_t)n_basis * n_basis * (l_is_complex ? 16 : 8)));
+  const int i_ph = in.add(phases, (size_t)n_omega * 16);
+  const int i_B = in.add(B, b_bytes);
+  const int i_L = in.add(L, (size_t)n_basis * n_basis * (l_is_complex ? 16 : 8));
+  FFB_TRY(in.upload());
   FFB_TRY(O.alloc(ctx, b_bytes));
-  FFB_TRY(ffbi_control_matrix_periodic(ctx, n_nops, n_basis, n_omega, repeats, ph.d(), Bd.d(),
-                                       Ld.d(), l_is_complex, O.as<double>()));
+  FFB_TRY(ffbi_control_matrix_periodic(ctx, n_nops, n_basis, n_omega, repeats, in.d(i_ph), in.d(i_B),
+                                       in.d(i_L), l_is_complex, O.as<double>()));
   FFB_TRY(ffb_d2h(ctx, out, O.p, b_bytes));
   FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return FFB_OK;
@@ -1078,21 +1095,18 @@ int ffb_infidelity(ffb_ctx* ctx, int n_lead, int n_nops, int n_sel, const int* i
   for (int i = 0; i < n_sel; ++i)
     FFB_REQUIRE(ctx, idx[i] >= 0 && idx[i] < n_nops, "infidelity: idx[%d]=%d out of range", i, idx[i]);
   DevBuf res;
-  const size_t s_elems = (spectrum_ndim == 1 ? 1 : spectrum_ndim == 2 ? (size_t)n_sel
-                                                                       : (size_t)n_sel * n_sel) * n_omega;
-  // one packed upload for the four inputs (a filter function that is still mirrored on the device --
-  // the pulse's cached array -- is not sent at all)
+  // a filter function that is still mirrored on the device (the pulse's cached array) is not sent at all
   PackedUpload in(ctx);
   const int i_F = in.add(F, (size_t)n_lead * n_nops * n_nops * n_omega * 16);
-  const int i_S = in.add(spectrum, s_elems * (spectrum_is_complex ? 16 : 8));
+  const int i_S = in.add(spectrum,
+                         spectrum_elems(spectrum_ndim, n_sel, n_omega) * (spectrum_is_complex ? 16 : 8));
   const int i_om = in.add(omega, (size_t)n_omega * 8);
   const int i_ix = in.add(idx, (size_t)n_sel * sizeof(int));
-  FFB_TRY(in.upload(ctx));
+  FFB_TRY(in.upload());
   const size_t n_out = (size_t)n_lead * (spectrum_ndim == 3 ? (size_t)n_sel * n_sel : n_sel);
   FFB_TRY(res.alloc(ctx, n_out * 8));
-  FFB_TRY(ffbi_infidelity(ctx, n_lead, n_nops, n_sel, reinterpret_cast<const int*>(in.d(i_ix)), n_omega,
-                          in.d(i_F), in.d(i_S), spectrum_ndim, spectrum_is_complex, in.d(i_om), d,
-                          res.as<double>()));
+  FFB_TRY(ffbi_infidelity(ctx, n_lead, n_nops, n_sel, in.d<int>(i_ix), n_omega, in.d(i_F), in.d(i_S),
+                          spectrum_ndim, spectrum_is_complex, in.d(i_om), d, res.as<double>()));
   FFB_TRY(ffb_d2h(ctx, out, res.p, n_out * 8));
   FFB_TRY(ffbi_comm_fetch_error(ctx));
   FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1146,9 +1160,9 @@ int ffb_infidelity_derivative(ffb_ctx* ctx, int G, int d, int n_cops, int n_nops
   const int i_B = control_matrix ? in.add(control_matrix, (size_t)n_nops * n_basis * n_omega * 16) : -1;
   const int i_ci = in.add(ctrl_idx, (size_t)n_ctrl * sizeof(int));
   const int i_si = in.add(sel_idx, (size_t)n_sel * sizeof(int));
-  const int i_sp = in.add(spectrum, (size_t)(spectrum_ndim == 2 ? n_sel : 1) * n_omega * 8);
+  const int i_sp = in.add(spectrum, spectrum_elems(spectrum_ndim, n_sel, n_omega) * 8);
   const int i_dp = n_coeffs_deps ? in.add(n_coeffs_deps, (size_t)n_nops * n_ctrl * G * 8) : -1;
-  FFB_TRY(in.upload(ctx));
+  FFB_TRY(in.upload());
   DevBuf ev, V, Q, B, res;
   const double *ev_d, *V_d, *Q_d;
   if (diag) {
@@ -1169,20 +1183,17 @@ int ffb_infidelity_derivative(ffb_ctx* ctx, int G, int d, int n_cops, int n_nops
   if (control_matrix) {
     B_d = in.d(i_B);
   } else {
-    const int herm = (all_hermitian(n_opers, n_nops, d) ? FFB_HERM_NOPERS : 0) |
-                     basis_flags(basis, n_basis, d);
     FFB_TRY(B.alloc(ctx, (size_t)n_nops * n_basis * n_omega * 16));
     FFB_TRY(ffbi_control_matrix(ctx, G, d, n_nops, n_basis, n_omega, ev_d, V_d, Q_d, in.d(i_om),
-                                in.d(i_bs), in.d(i_no), in.d(i_nc), in.d(i_dt), in.d(i_ts), herm,
-                                B.as<double>()));
+                                in.d(i_bs), in.d(i_no), in.d(i_nc), in.d(i_dt), in.d(i_ts),
+                                herm_flags(n_opers, n_nops, basis, n_basis, d), B.as<double>()));
     B_d = B.as<double>();
   }
   const size_t n_out = (size_t)n_sel * G * n_ctrl;
   FFB_TRY(res.alloc(ctx, n_out * 8));
   FFB_TRY(ffbi_infidelity_derivative(
       ctx, G, d, n_nops, n_basis, n_omega, ev_d, V_d, Q_d, in.d(i_om), in.d(i_bs), in.d(i_no),
-      in.d(i_nc), in.d(i_dt), in.d(i_ts), in.d(i_co), B_d, n_ctrl,
-      reinterpret_cast<const int*>(in.d(i_ci)), n_sel, reinterpret_cast<const int*>(in.d(i_si)),
+      in.d(i_nc), in.d(i_dt), in.d(i_ts), in.d(i_co), B_d, n_ctrl, in.d<int>(i_ci), n_sel, in.d<int>(i_si),
       in.d(i_sp), spectrum_ndim, n_coeffs_deps ? in.d(i_dp) : nullptr, norm_d, res.as<double>()));
   FFB_TRY(ffb_d2h(ctx, out, res.p, n_out * 8));
   if (diag) FFB_TRY(ffb_conv_fetch(ctx));
@@ -1202,18 +1213,19 @@ int ffb_decay_amplitudes(ffb_ctx* ctx, int P, int n_nops, int n_sel, const int* 
   for (int i = 0; i < n_sel; ++i)
     FFB_REQUIRE(ctx, idx[i] >= 0 && idx[i] < n_nops, "decay amplitudes: idx[%d]=%d out of range", i,
                 idx[i]);
-  Upload Bd, Sd, Od, Id;
+  PackedUpload in(ctx);
   DevBuf res;
+  const int i_B = in.add(B, (size_t)P * n_nops * n_basis * n_omega * 16);
+  const int i_S = in.add(spectrum,
+                         spectrum_elems(spectrum_ndim, n_sel, n_omega) * (spectrum_is_complex ? 16 : 8));
+  const int i_om = in.add(omega, (size_t)n_omega * 8);
+  const int i_ix = in.add(idx, (size_t)n_sel * sizeof(int));
+  FFB_TRY(in.upload());
   const size_t n_pairs = spectrum_ndim == 3 ? (size_t)n_sel * n_sel : n_sel;
-  const size_t s_elems = (spectrum_ndim == 1 ? 1 : n_pairs) * n_omega;
-  FFB_TRY(Bd.put(ctx, B, (size_t)P * n_nops * n_basis * n_omega * 16));
-  FFB_TRY(Sd.put(ctx, spectrum, s_elems * (spectrum_is_complex ? 16 : 8)));
-  FFB_TRY(Od.put(ctx, omega, (size_t)n_omega * 8));
-  FFB_TRY(Id.put(ctx, idx, (size_t)n_sel * sizeof(int)));
   const size_t n_out = (size_t)P * P * n_pairs * n_basis * n_basis;
   FFB_TRY(res.alloc(ctx, n_out * 8));
-  FFB_TRY(ffbi_decay_amplitudes(ctx, P, n_nops, n_sel, Id.buf.as<int>(), n_basis, n_omega, Bd.d(),
-                                Sd.d(), spectrum_ndim, spectrum_is_complex, Od.d(),
+  FFB_TRY(ffbi_decay_amplitudes(ctx, P, n_nops, n_sel, in.d<int>(i_ix), n_basis, n_omega, in.d(i_B),
+                                in.d(i_S), spectrum_ndim, spectrum_is_complex, in.d(i_om),
                                 res.as<double>()));
   FFB_TRY(ffb_d2h(ctx, out, res.p, n_out * 8));
   FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1259,13 +1271,11 @@ int ffb_concatenate_many(ffb_ctx* ctx, int n_seq, int L, int n_lib, int d, int n
   if (infidelity) {
     FFB_REQUIRE(ctx, spectrum_ndim >= 1 && spectrum_ndim <= 3, "concatenate_many: spectrum_ndim=%d",
                 spectrum_ndim);
-    const size_t s_elems = (spectrum_ndim == 1 ? 1 : spectrum_ndim == 2 ? (size_t)n_nops
-                                                                         : (size_t)n_nops * n_nops) * n_omega;
-    i_sp = in.add(spectrum, s_elems * (spectrum_is_complex ? 16 : 8));
+    i_sp = in.add(spectrum, spectrum_elems(spectrum_ndim, n_nops, n_omega) * (spectrum_is_complex ? 16 : 8));
     n_inf = (size_t)n_seq * (spectrum_ndim == 3 ? (size_t)n_nops * n_nops : n_nops);
   }
   if (total_propagator_liouville) i_bs = in.add(basis, (size_t)n_basis * dd * 16);
-  FFB_TRY(in.upload(ctx));
+  FFB_TRY(in.upload());
   const size_t b_bytes = (size_t)n_seq * n_nops * n_basis * n_omega * 16;
   const size_t f_bytes = (size_t)n_seq * n_nops * n_nops * n_omega * 16;
   const bool need_F = filter_function || infidelity;
@@ -1277,9 +1287,8 @@ int ffb_concatenate_many(ffb_ctx* ctx, int n_seq, int L, int n_lib, int d, int n
   const int o_F = need_F ? out.add(filter_function, f_bytes) : -1;
   const int o_I = infidelity ? out.add(infidelity, n_inf * 8) : -1;
   FFB_TRY(out.alloc(ctx));
-  FFB_TRY(ffbi_concatenate_many(ctx, n_seq, L, d, n_nops, n_basis, n_omega,
-                                reinterpret_cast<const int*>(in.d(i_ix)), in.d(i_lb), in.d(i_lp),
-                                in.d(i_ll), in.d(i_lu), out.d(o_U), out.d(o_B),
+  FFB_TRY(ffbi_concatenate_many(ctx, n_seq, L, d, n_nops, n_basis, n_omega, in.d<int>(i_ix), in.d(i_lb),
+                                in.d(i_lp), in.d(i_ll), in.d(i_lu), out.d(o_U), out.d(o_B),
                                 need_F ? out.d(o_F) : nullptr));
   if (infidelity)
     FFB_TRY(ffbi_infidelity(ctx, n_seq, n_nops, n_nops, nullptr, n_omega, out.d(o_F), in.d(i_sp),
@@ -1315,11 +1324,7 @@ int ffb_concatenate_pulses(ffb_ctx* ctx, int P, int d, int n_nops, int n_basis, 
   FFB_REQUIRE(ctx, filter_function_kind >= 0 && filter_function_kind <= 2 &&
                        (filter_function_kind == 0 || filter_function),
               "concatenate_pulses: filter_function_kind=%d", filter_function_kind);
-  static const bool trace = getenv("FFB_TRACE") && atoi(getenv("FFB_TRACE")) != 0;
-  const auto t_enter = std::chrono::steady_clock::now();
-  auto since = [&]() {
-    return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - t_enter).count();
-  };
+  const TraceClock since;
   const int64_t hits0 = ctx->shadow_hits;
   const bool keep_shadow = ctx->shadow_next;
   ctx->shadow_next = false;
@@ -1334,12 +1339,45 @@ int ffb_concatenate_pulses(ffb_ctx* ctx, int P, int d, int n_nops, int n_basis, 
       FFB_REQUIRE(ctx, row_of[(size_t)p * n_nops + j] < 0 || cached[p],
                   "concatenate_pulses: pulse %d has cached rows but no array", p);
 
-  Upload om, bs, ph, Qd;
-  FFB_TRY(om.put(ctx, omega, (size_t)n_omega * 8));
-  FFB_TRY(bs.put(ctx, basis, (size_t)n_basis * dd * 16));
-  if (P > 1) {
-    FFB_TRY(ph.put(ctx, phases, (size_t)(P - 1) * n_omega * 16));
-    FFB_TRY(Qd.put(ctx, liouville, (size_t)(P - 1) * n_basis * n_basis * 8));
+  // every input in one packed upload, before any launch: omega, the basis, the contraction's phases and
+  // Liouville propagators, and for each pulse with missing rows its eigensystem, time steps and the
+  // noise operators and coefficients of those rows (seven parts from fill[p] on, in the order
+  // ffbi_control_matrix takes them)
+  PackedUpload in(ctx);
+  const int i_om = in.add(omega, (size_t)n_omega * 8);
+  const int i_bs = in.add(basis, (size_t)n_basis * dd * 16);
+  const int i_ph = P > 1 ? in.add(phases, (size_t)(P - 1) * n_omega * 16) : -1;
+  const int i_Q = P > 1 ? in.add(liouville, (size_t)(P - 1) * n_basis * n_basis * 8) : -1;
+  std::vector<std::vector<int>> missing_rows(P);
+  std::vector<int> fill(P, -1), herm(P, 0);
+  {
+    std::vector<std::vector<double>> keep;  // host staging of the subsets, read by in.upload()
+    for (int p = 0; p < P; ++p) {
+      std::vector<int>& missing = missing_rows[p];
+      for (int j = 0; j < n_nops; ++j)
+        if (row_of[(size_t)p * n_nops + j] < 0) missing.push_back(j);
+      if (missing.empty()) continue;
+      const int m = (int)missing.size(), Gp = G[p];
+      FFB_REQUIRE(ctx, Gp >= 1 && eigvals[p] && eigvecs[p] && propagators[p] && dt[p] && t[p] &&
+                           n_coeffs[p], "concatenate_pulses: pulse %d lacks its diagonalisation", p);
+      keep.emplace_back((size_t)m * dd * 2);
+      keep.emplace_back((size_t)m * Gp);
+      std::vector<double>& ops = keep[keep.size() - 2];
+      std::vector<double>& cf = keep[keep.size() - 1];
+      for (int i = 0; i < m; ++i) {
+        std::memcpy(ops.data() + (size_t)i * dd * 2, n_opers + (size_t)missing[i] * dd * 2, dd * 16);
+        std::memcpy(cf.data() + (size_t)i * Gp, n_coeffs[p] + (size_t)missing[i] * Gp, (size_t)Gp * 8);
+      }
+      herm[p] = (all_hermitian(ops.data(), m, d) ? FFB_HERM_NOPERS : 0) | (basis_herm ? FFB_HERM_BASIS : 0);
+      fill[p] = in.add(eigvals[p], (size_t)Gp * d * 8);
+      in.add(eigvecs[p], (size_t)Gp * dd * 16);
+      in.add(propagators[p], (size_t)Gp * dd * 16);
+      in.add(ops.data(), (size_t)m * dd * 16);
+      in.add(cf.data(), (size_t)m * Gp * 8);
+      in.add(dt[p], (size_t)Gp * 8);
+      in.add(t[p], (size_t)(Gp + 1) * 8);
+    }
+    FFB_TRY(in.upload());
   }
   // Full stack (P pulse slots) when it takes at most a quarter of the device memory: all from-scratch
   // fills are enqueued first, the cached rows are uploaded on the copy stream WHILE the fills run, and
@@ -1353,12 +1391,9 @@ int ffb_concatenate_pulses(ffb_ctx* ctx, int P, int d, int n_nops, int n_basis, 
   DevBuf stack, scratch, result;
   FFB_TRY(stack.alloc(ctx, (size_t)slots * pulse_bytes));
   if (full_stack) FFB_TRY(result.alloc(ctx, (size_t)(correlations ? P : 1) * pulse_bytes));
-  if (full_stack && !ctx->copy_stream) {
-    FFB_TRY(ensure_copy_stream(ctx));
-  }
   if (full_stack) {  // the copy stream must not touch pool memory before earlier work is done with it
-    FFB_CUDA(ctx, cudaEventRecord(ctx->copy_ev[0], ctx->stream));
-    FFB_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_ev[0], 0));
+    FFB_TRY(ensure_copy_stream(ctx));
+    FFB_TRY(after(ctx, 0, ctx->stream, ctx->copy_stream));
   }
   cudaStream_t up_stream = full_stack ? ctx->copy_stream : ctx->stream;
 
@@ -1382,38 +1417,13 @@ int ffb_concatenate_pulses(ffb_ctx* ctx, int P, int d, int n_nops, int n_basis, 
     return FFB_OK;
   };
 
-  std::vector<std::vector<double>> keep;  // host staging that must outlive the async uploads
-  std::vector<int> missing;
   for (int p = 0; p < P; ++p) {
     const int slot = full_stack ? p : std::min(p, 1);
     char* dst = stack.as<char>() + (size_t)slot * pulse_bytes;
-    const int* rows = row_of + (size_t)p * n_nops;
-    missing.clear();
-    for (int j = 0; j < n_nops; ++j)
-      if (rows[j] < 0) missing.push_back(j);
     if (!full_stack) FFB_TRY(upload_cached(p, dst));
+    const std::vector<int>& missing = missing_rows[p];
     if (!missing.empty()) {
-      const int m = (int)missing.size(), Gp = G[p];
-      FFB_REQUIRE(ctx, Gp >= 1 && eigvals[p] && eigvecs[p] && propagators[p] && dt[p] && t[p] &&
-                           n_coeffs[p], "concatenate_pulses: pulse %d lacks its diagonalisation", p);
-      keep.emplace_back((size_t)m * dd * 2);
-      keep.emplace_back((size_t)m * Gp);
-      std::vector<double>& ops = keep[keep.size() - 2];
-      std::vector<double>& cf = keep[keep.size() - 1];
-      for (int i = 0; i < m; ++i) {
-        std::memcpy(ops.data() + (size_t)i * dd * 2, n_opers + (size_t)missing[i] * dd * 2, dd * 16);
-        std::memcpy(cf.data() + (size_t)i * Gp, n_coeffs[p] + (size_t)missing[i] * Gp, (size_t)Gp * 8);
-      }
-      const int herm = (all_hermitian(ops.data(), m, d) ? FFB_HERM_NOPERS : 0) |
-                       (basis_herm ? FFB_HERM_BASIS : 0);
-      Upload ev, V, Qp, no, nc, dts, ts;
-      FFB_TRY(ev.put(ctx, eigvals[p], (size_t)Gp * d * 8));
-      FFB_TRY(V.put(ctx, eigvecs[p], (size_t)Gp * dd * 16));
-      FFB_TRY(Qp.put(ctx, propagators[p], (size_t)Gp * dd * 16));
-      FFB_TRY(no.put(ctx, ops.data(), (size_t)m * dd * 16));
-      FFB_TRY(nc.put(ctx, cf.data(), (size_t)m * Gp * 8));
-      FFB_TRY(dts.put(ctx, dt[p], (size_t)Gp * 8));
-      FFB_TRY(ts.put(ctx, t[p], (size_t)(Gp + 1) * 8));
+      const int m = (int)missing.size(), i0 = fill[p];
       // one contiguous run of missing rows is written in place, otherwise through scratch
       const bool contiguous = missing.back() - missing.front() + 1 == m;
       double* target = reinterpret_cast<double*>(dst + (size_t)missing.front() * row_bytes);
@@ -1421,8 +1431,9 @@ int ffb_concatenate_pulses(ffb_ctx* ctx, int P, int d, int n_nops, int n_basis, 
         FFB_TRY(scratch.alloc(ctx, (size_t)m * row_bytes));
         target = scratch.as<double>();
       }
-      FFB_TRY(ffbi_control_matrix(ctx, Gp, d, m, n_basis, n_omega, ev.d(), V.d(), Qp.d(), om.d(),
-                                  bs.d(), no.d(), nc.d(), dts.d(), ts.d(), herm, target));
+      FFB_TRY(ffbi_control_matrix(ctx, G[p], d, m, n_basis, n_omega, in.d(i0), in.d(i0 + 1), in.d(i0 + 2),
+                                  in.d(i_om), in.d(i_bs), in.d(i0 + 3), in.d(i0 + 4), in.d(i0 + 5),
+                                  in.d(i0 + 6), herm[p], target));
       if (!contiguous) {
         for (int i = 0; i < m; ++i) {
           int run = 1;
@@ -1436,8 +1447,8 @@ int ffb_concatenate_pulses(ffb_ctx* ctx, int P, int d, int n_nops, int n_basis, 
       }
     }
     if (!full_stack && p >= 1) {
-      FFB_TRY(ffbi_from_atomic(ctx, 2, n_nops, n_basis, n_omega, ph.d() + (size_t)(p - 1) * n_omega * 2,
-                               stack.as<double>(), Qd.d() + (size_t)(p - 1) * n_basis * n_basis, 0, 0,
+      FFB_TRY(ffbi_from_atomic(ctx, 2, n_nops, n_basis, n_omega, in.d(i_ph) + (size_t)(p - 1) * n_omega * 2,
+                               stack.as<double>(), in.d(i_Q) + (size_t)(p - 1) * n_basis * n_basis, 0, 0,
                                stack.as<double>()));
     }
   }
@@ -1447,8 +1458,7 @@ int ffb_concatenate_pulses(ffb_ctx* ctx, int P, int d, int n_nops, int n_basis, 
     // cached rows: issued after the fills were enqueued, so that even a pageable source (staged by the
     // driver while the host thread waits) overlaps them
     for (int p = 0; p < P; ++p) FFB_TRY(upload_cached(p, stack.as<char>() + (size_t)p * pulse_bytes));
-    FFB_CUDA(ctx, cudaEventRecord(ctx->copy_ev[1], ctx->copy_stream));
-    FFB_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->copy_ev[1], 0));
+    FFB_TRY(after(ctx, 1, ctx->copy_stream, ctx->stream));
     B_dev = result.as<double>();
     // total control matrix: a few row chunks, each downloaded on the copy stream while the next one
     // is computed (the download of the whole result takes about as long as computing it)
@@ -1457,11 +1467,10 @@ int ffb_concatenate_pulses(ffb_ctx* ctx, int P, int d, int n_nops, int n_basis, 
       const int j0 = (int)((long long)c * n_nops / n_chunks);
       const int j1 = (int)((long long)(c + 1) * n_nops / n_chunks);
       FFB_TRY(ffbi_from_atomic_rows(ctx, P, n_nops, j0, j1 - j0, n_basis, n_omega,
-                                    P > 1 ? ph.d() : nullptr, stack.as<double>(),
-                                    P > 1 ? Qd.d() : nullptr, 0, correlations, result.as<double>()));
+                                    P > 1 ? in.d(i_ph) : nullptr, stack.as<double>(),
+                                    P > 1 ? in.d(i_Q) : nullptr, 0, correlations, result.as<double>()));
       if (n_chunks > 1) {
-        FFB_CUDA(ctx, cudaEventRecord(ctx->copy_ev[0], ctx->stream));
-        FFB_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_ev[0], 0));
+        FFB_TRY(after(ctx, 0, ctx->stream, ctx->copy_stream));
         FFB_CUDA(ctx, cudaMemcpyAsync(reinterpret_cast<char*>(control_matrix) + (size_t)j0 * row_bytes,
                                       reinterpret_cast<const char*>(B_dev) + (size_t)j0 * row_bytes,
                                       (size_t)(j1 - j0) * row_bytes, cudaMemcpyDeviceToHost,
@@ -1480,8 +1489,7 @@ int ffb_concatenate_pulses(ffb_ctx* ctx, int P, int d, int n_nops, int n_basis, 
   }
   if (control_matrix && full_stack && filter_function_kind) {
     // download the control matrix on the copy stream while the filter function is computed
-    FFB_CUDA(ctx, cudaEventRecord(ctx->copy_ev[0], ctx->stream));
-    FFB_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_ev[0], 0));
+    FFB_TRY(after(ctx, 0, ctx->stream, ctx->copy_stream));
     FFB_CUDA(ctx, cudaMemcpyAsync(control_matrix, B_dev, (size_t)lead * pulse_bytes,
                                   cudaMemcpyDeviceToHost, ctx->copy_stream));
   } else if (control_matrix) {
@@ -1496,7 +1504,7 @@ int ffb_concatenate_pulses(ffb_ctx* ctx, int P, int d, int n_nops, int n_basis, 
   if (full_stack) FFB_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream));
   const double us_copy = since();
   FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if (trace)
+  if (ffb_trace())
     fprintf(stderr, "[ffb trace] concatenate_pulses: P=%d, fills enqueued %.0f us, all enqueued %.0f us, "
             "copy stream done %.0f us, main stream done %.0f us; %lld cached row runs read from device "
             "shadows; %s stack\n", P, us_fills, us_enqueued, us_copy, since(),
@@ -1515,14 +1523,15 @@ int ffb_liouville_representation(ffb_ctx* ctx, int n, int d, int n_basis, const 
   FFB_TRY(enter(ctx));
   FFB_REQUIRE(ctx, U && basis && out, "liouville: null pointer");
   FFB_REQUIRE(ctx, n >= 1 && d >= 1 && n_basis >= 1, "liouville: bad shape");
-  Upload Ud, Bd;
+  PackedUpload in(ctx);
   DevBuf O;
   const size_t dd = (size_t)d * d;
-  FFB_TRY(Ud.put(ctx, U, (size_t)n * dd * 16));
-  FFB_TRY(Bd.put(ctx, basis, (size_t)n_basis * dd * 16));
+  const int i_U = in.add(U, (size_t)n * dd * 16);
+  const int i_bs = in.add(basis, (size_t)n_basis * dd * 16);
+  FFB_TRY(in.upload());
   const size_t out_bytes = (size_t)n * n_basis * n_basis * 16;
   FFB_TRY(O.alloc(ctx, out_bytes));
-  FFB_TRY(ffbi_liouville(ctx, n, d, n_basis, Ud.d(), Bd.d(), O.as<double>()));
+  FFB_TRY(ffbi_liouville(ctx, n, d, n_basis, in.d(i_U), in.d(i_bs), O.as<double>()));
   FFB_TRY(ffb_d2h(ctx, out, O.p, out_bytes));
   FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return FFB_OK;
@@ -1531,11 +1540,12 @@ int ffb_liouville_representation(ffb_ctx* ctx, int n, int d, int n_basis, const 
 int ffb_cexp(ffb_ctx* ctx, int n, const double* x, double scale, double* out) {
   FFB_TRY(enter(ctx));
   FFB_REQUIRE(ctx, x && out && n >= 1, "cexp: bad arguments");
-  Upload xd;
+  PackedUpload in(ctx);
   DevBuf O;
-  FFB_TRY(xd.put(ctx, x, (size_t)n * 8));
+  const int i_x = in.add(x, (size_t)n * 8);
+  FFB_TRY(in.upload());
   FFB_TRY(O.alloc(ctx, (size_t)n * 16));
-  FFB_TRY(ffbi_cexp(ctx, n, xd.d(), scale, O.as<double>()));
+  FFB_TRY(ffbi_cexp(ctx, n, in.d(i_x), scale, O.as<double>()));
   FFB_TRY(ffb_d2h(ctx, out, O.p, (size_t)n * 16));
   FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return FFB_OK;
@@ -1544,11 +1554,12 @@ int ffb_cexp(ffb_ctx* ctx, int n, const double* x, double scale, double* out) {
 int ffb_cexpm1(ffb_ctx* ctx, int n, const double* x, double* out) {
   FFB_TRY(enter(ctx));
   FFB_REQUIRE(ctx, x && out && n >= 1, "cexpm1: bad arguments");
-  Upload xd;
+  PackedUpload in(ctx);
   DevBuf O;
-  FFB_TRY(xd.put(ctx, x, (size_t)n * 8));
+  const int i_x = in.add(x, (size_t)n * 8);
+  FFB_TRY(in.upload());
   FFB_TRY(O.alloc(ctx, (size_t)n * 16));
-  FFB_TRY(ffbi_cexpm1(ctx, n, xd.d(), O.as<double>()));
+  FFB_TRY(ffbi_cexpm1(ctx, n, in.d(i_x), O.as<double>()));
   FFB_TRY(ffb_d2h(ctx, out, O.p, (size_t)n * 16));
   FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return FFB_OK;
@@ -1573,19 +1584,14 @@ int ffb_pulse_filter_function(ffb_ctx* ctx, int G, int d, int n_cops, int n_nops
   const bool keep = ctx->shadow_next;
   ctx->shadow_next = false;
   const size_t dd = (size_t)d * d;
-  const int herm = (all_hermitian(n_opers, n_nops, d) ? FFB_HERM_NOPERS : 0) |
-                   basis_flags(basis, n_basis, d);
+  const int herm = herm_flags(n_opers, n_nops, basis, n_basis, d);
   FFB_TRY(ensure_copy_stream(ctx));
   // FFB_TRACE=1: host-side timestamps of the pipeline stages on stderr (where does e2e time go?)
-  static const bool trace = getenv("FFB_TRACE") && atoi(getenv("FFB_TRACE")) != 0;
-  const auto t_enter = std::chrono::steady_clock::now();
-  auto since = [&]() {
-    return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - t_enter).count();
-  };
+  const TraceClock since;
   double us_packed = 0, us_enqueued = 0, us_main = 0;
   std::string marks;
   auto mark = [&](const char* what) {
-    if (!trace) return;
+    if (!ffb_trace()) return;
     char buf[64];
     snprintf(buf, sizeof(buf), " %s@%.0f", what, since());
     marks += buf;
@@ -1616,12 +1622,10 @@ int ffb_pulse_filter_function(ffb_ctx* ctx, int G, int d, int n_cops, int n_nops
   if (infidelity) {
     FFB_REQUIRE(ctx, spectrum_ndim >= 1 && spectrum_ndim <= 3, "pulse pipeline: spectrum_ndim=%d",
                 spectrum_ndim);
-    const size_t s_elems = (spectrum_ndim == 1 ? 1 : spectrum_ndim == 2 ? (size_t)n_nops
-                                                                         : (size_t)n_nops * n_nops) * n_omega;
-    i_sp = in.add(spectrum, s_elems * (spectrum_is_complex ? 16 : 8));
+    i_sp = in.add(spectrum, spectrum_elems(spectrum_ndim, n_nops, n_omega) * (spectrum_is_complex ? 16 : 8));
     n_inf = spectrum_ndim == 3 ? (size_t)n_nops * n_nops : n_nops;
   }
-  FFB_TRY(in.upload(ctx));
+  FFB_TRY(in.upload());
   us_packed = since();
   const size_t b_bytes = (size_t)n_nops * n_basis * n_omega * 16;
   const size_t f_bytes = (size_t)n_nops * n_nops * n_omega * 16;
@@ -1655,8 +1659,7 @@ int ffb_pulse_filter_function(ffb_ctx* ctx, int G, int d, int n_cops, int n_nops
   const size_t out_bytes = (control_matrix ? b_bytes : 0) + (filter_function ? f_bytes : 0);
   const bool overlap = early_bytes + out_bytes >= ((size_t)256 << 10);
   if (overlap) {
-    FFB_CUDA(ctx, cudaEventRecord(ctx->copy_ev[0], ctx->stream));
-    FFB_CUDA(ctx, cudaStreamWaitEvent(cs, ctx->copy_ev[0], 0));
+    FFB_TRY(after(ctx, 0, ctx->stream, cs));
     FFB_TRY(out.download(ctx, {o_ev, o_V, o_Q, o_ph, o_li}, cs));
   }
 
@@ -1666,22 +1669,15 @@ int ffb_pulse_filter_function(ffb_ctx* ctx, int G, int d, int n_cops, int n_nops
   // 105 MB, 1.9 ms at 56 GB/s)
   FreqBlocks fb;
   fb.n_blocks = pipeline_blocks(out_bytes, n_omega);
-  const size_t pitch = (size_t)n_omega * 16;
   fb.after_block = [&](int w0, int w1) -> int {
-    const size_t off = (size_t)w0 * 16, width = (size_t)(w1 - w0) * 16;
     FFB_TRY(ffbi_filter_function_ld(ctx, 1, n_nops, n_basis, w1 - w0, (size_t)n_omega,
                                     out.d(o_B) + 2 * (size_t)w0, out.d(o_F) + 2 * (size_t)w0));
     if (fb.n_blocks == 1) return FFB_OK;  // one block: whole arrays, copied below
-    FFB_CUDA(ctx, cudaEventRecord(ctx->copy_ev[1], ctx->stream));
-    FFB_CUDA(ctx, cudaStreamWaitEvent(cs, ctx->copy_ev[1], 0));
+    FFB_TRY(after(ctx, 1, ctx->stream, cs));
     if (control_matrix)
-      FFB_CUDA(ctx, cudaMemcpy2DAsync(reinterpret_cast<char*>(control_matrix) + off, pitch,
-                                      out.d<char>(o_B) + off, pitch, width,
-                                      (size_t)n_nops * n_basis, cudaMemcpyDeviceToHost, cs));
+      FFB_TRY(download_freqs(ctx, control_matrix, out.d(o_B), (size_t)n_nops * n_basis, n_omega, w0, w1));
     if (filter_function)
-      FFB_CUDA(ctx, cudaMemcpy2DAsync(reinterpret_cast<char*>(filter_function) + off, pitch,
-                                      out.d<char>(o_F) + off, pitch, width,
-                                      (size_t)n_nops * n_nops, cudaMemcpyDeviceToHost, cs));
+      FFB_TRY(download_freqs(ctx, filter_function, out.d(o_F), (size_t)n_nops * n_nops, n_omega, w0, w1));
     return FFB_OK;
   };
   FFB_TRY(ffbi_control_matrix(ctx, G, d, n_nops, n_basis, n_omega, out.d(o_ev), out.d(o_V),
@@ -1689,8 +1685,7 @@ int ffb_pulse_filter_function(ffb_ctx* ctx, int G, int d, int n_cops, int n_nops
                               in.d(i_dt), in.d(i_ts), herm, out.d(o_B), &fb));
   mark("ctrlmat");
   if (overlap && fb.n_blocks == 1) {  // B and F in one copy while the integral runs
-    FFB_CUDA(ctx, cudaEventRecord(ctx->copy_ev[1], ctx->stream));
-    FFB_CUDA(ctx, cudaStreamWaitEvent(cs, ctx->copy_ev[1], 0));
+    FFB_TRY(after(ctx, 1, ctx->stream, cs));
     FFB_TRY(out.download(ctx, {o_B, o_F}, cs));
   }
   if (infidelity)
@@ -1711,7 +1706,7 @@ int ffb_pulse_filter_function(ffb_ctx* ctx, int G, int d, int n_cops, int n_nops
   out.finish(ctx);
   FFB_TRY(ffb_conv_check(ctx));
   FFB_TRY(ffbi_comm_check_error(ctx));
-  if (trace)
+  if (ffb_trace())
     fprintf(stderr, "[ffb trace] pulse pipeline: inputs packed+upload enqueued %.0f us, all work enqueued "
             "%.0f us, main stream done %.0f us, copy stream done %.0f us;%s\n", us_packed, us_enqueued,
             us_main, since(), marks.c_str());

@@ -58,10 +58,10 @@ struct ffb_ctx {
   cudaStream_t stream = nullptr;  // the stream work is enqueued on (own or external)
   std::string err;
   int64_t launches = 0;
-  // second stream for bulk host<->device copies that overlap kernels (ffb_concatenate_pulses);
-  // ordered against `stream` with the two events
   // 256-entry table of (sin, cos)(k pi / 128) for the table-driven sincos of the control-matrix kernels
   double* trig_table = nullptr;
+  // second stream for bulk host<->device copies that overlap kernels (the pulse pipeline, the control
+  // matrix, ffb_concatenate_pulses); ordered against `stream` with the two events
   cudaStream_t copy_stream = nullptr;
   cudaEvent_t copy_ev[2] = {nullptr, nullptr};
   // page-locked staging block: the small host inputs of a call are packed here and uploaded by ONE copy
@@ -128,6 +128,8 @@ struct ffb_ctx {
 };
 
 int ffb_fail(ffb_ctx* ctx, int code, const char* fmt, ...);
+// FFB_TRACE set and nonzero (read once): host-side timelines and dispatch lines on stderr
+bool ffb_trace();
 
 #define FFB_CUDA(ctx, expr)                                                                    \
   do {                                                                                         \

@@ -2021,7 +2021,7 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
   // block boundaries on multiples of 64 frequencies (the frequency tiles of all kernel variants)
   const int n_blocks = blocks ? std::max(1, std::min(blocks->n_blocks, ceil_div(n_omega_all, 64))) : 1;
   const int per_block = ceil_div(ceil_div(n_omega_all, n_blocks), 64) * 64;
-  const bool trace = getenv("FFB_TRACE") != nullptr;
+  const bool trace = ffb_trace();
   for (int w0 = 0; w0 < n_omega_all; w0 += per_block) {
     const int w1 = std::min(n_omega_all, w0 + per_block);
     ffb_dispatch_record disp = {};
