@@ -23,23 +23,9 @@
 #include <cstdlib>
 
 #include "ffb_common.cuh"
+#include "ffb_device.cuh"
 
 namespace {
-
-__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
-  asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-      : "+d"(c0), "+d"(c1)
-      : "d"(a), "d"(b));
-}
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
-  const unsigned s = (unsigned)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem_src));
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N));
-}
 
 // qstream[g][ls][s][lt][lane] = Q_g[4 s + lane % 4][(ls * LT + lt) * 8 + lane / 4]   (0 outside)
 __global__ void __launch_bounds__(256)

@@ -45,6 +45,8 @@
 #include <cstdlib>
 
 #include "ffb_common.cuh"
+#include "ffb_device.cuh"
+#include "ffb_phase.cuh"
 
 
 namespace {
@@ -52,55 +54,6 @@ namespace {
 // ------------------------------------------------------------------------------------------------
 // math helpers
 // ------------------------------------------------------------------------------------------------
-// sin/cos with a Cody-Waite reduction.  fma keeps x - k*pi/2 accurate to ~1e-16 ABSOLUTE,
-// which is what a unit-modulus phase factor needs (CUDA's sincos switches to Payne-Hanek above 1e5
-// to keep the RELATIVE error near zeros of sin, which is irrelevant here).  Branch free.  Verified
-// against sincos() on B200 up to |x| = 1e7 (max abs deviation 1.1e-16); beyond ~1e9 the rounding of
-// the argument itself (ulp(w t) > 1e-7 rad) has destroyed the phase in the reference too.
-// The constants live in constant memory so that they enter the DFMAs as c[bank][offset] operands: as
-// immediates each one costs two UMOV/IMAD.MOV issue slots per use (ncu: 53 of the 258 instructions per
-// warp and segment of the DFMA kernel), and 16 doubles are too many to pin in registers.
-__constant__ double SC_K[16] = {
-    6.36619772367581382433e-01,   // 0: 2/pi
-    6755399441055744.0,           // 1: 1.5 * 2^52, round-to-nearest-integer by addition
-    1.57079632679489655800e+00,   // 2: pi/2 high
-    6.12323399573676603587e-17,   // 3: pi/2 middle
-    1.58969099521155010221e-10,   // 4..9: sin polynomial
-    -2.50507602534068634195e-08, 2.75573137070700676789e-06, -1.98412698298579493134e-04,
-    8.33333333332248946124e-03, -1.66666666666666324348e-01,
-    -1.13596475577881948265e-11,  // 10..15: cos polynomial
-    2.08757232129817482790e-09, -2.75573143513906633035e-07, 2.48015872894767294178e-05,
-    -1.38888888888741095749e-03, 4.16666666666666019037e-02};
-
-__device__ __forceinline__ void sincos_cw(double x, double& sn, double& cs) {
-  double kd = fma(x, SC_K[0], SC_K[1]);
-  const int q = __double2loint(kd);
-  kd -= SC_K[1];
-  // two-constant Cody-Waite: the third term of pi/2 (1.5e-33 k) is below 1e-17 for |x| < 1e16
-  double r = fma(-kd, SC_K[2], x);
-  r = fma(-kd, SC_K[3], r);
-  const double r2 = r * r;
-  double ps = fma(r2, SC_K[4], SC_K[5]);
-  ps = fma(ps, r2, SC_K[6]);
-  ps = fma(ps, r2, SC_K[7]);
-  ps = fma(ps, r2, SC_K[8]);
-  ps = fma(ps, r2, SC_K[9]);
-  const double s = fma(r * r2, ps, r);
-  double pc = fma(r2, SC_K[10], SC_K[11]);
-  pc = fma(pc, r2, SC_K[12]);
-  pc = fma(pc, r2, SC_K[13]);
-  pc = fma(pc, r2, SC_K[14]);
-  pc = fma(pc, r2, SC_K[15]);
-  const double c = fma(r2 * r2, pc, fma(r2, -0.5, 1.0));
-  // quadrant: swap for odd q, flip signs through the sign bit (integer ops, not the FP64 pipe)
-  const double ss = (q & 1) ? c : s;
-  const double cc = (q & 1) ? s : c;
-  const int s_flip = (q & 2) << 30;        // bit 31 of the high word
-  const int c_flip = ((q + 1) & 2) << 30;
-  sn = __hiloint2double(__double2hiint(ss) ^ s_flip, __double2loint(ss));
-  cs = __hiloint2double(__double2hiint(cc) ^ c_flip, __double2loint(cc));
-}
-
 // Table-driven variant for the thread-per-frequency kernel: x = k pi/128 + r, |r| <= pi/256, so sin r
 // and cos r need three terms each (remainders r^7/5040 < 1e-17, r^8/40320 < 1e-20) and the quadrant
 // logic disappears into the 256-entry table (sin, cos)(k pi/128) held in shared memory:
@@ -119,76 +72,7 @@ __global__ void trig_table_kernel(double2* __restrict__ table) {
   table[k] = make_double2(sn, cs);
 }
 
-// 1/x to ~1 ulp: MUFU.RCP64H seed + two Newton steps on the FP64 pipe.
-__device__ __forceinline__ double rcp_nr(double x) {
-  double r;
-  asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(x));
-  double e = fma(-x, r, 1.0);
-  r = fma(r, e, r);
-  e = fma(-x, r, 1.0);
-  r = fma(r, e, r);
-  return r;
-}
-
-constexpr double SQRT2 = 1.41421356237309504880;
-// |sqrt(2) sin(x dt / 2)| below 2^-10 sqrt(2) -> direct evaluation (SMALL_SIN_HI, compared on the high word)
 constexpr double TINY_OMEGA = 1e-290;               // |w| below this is treated as the exact zero
-
-// I(x) = (e^{i x dt} - 1) / (i x) evaluated directly with the rounding sequence of numeric.py:156-165
-// (y = x * dt); = dt for x == 0.  Only used by the rare fix-up path.
-__device__ __forceinline__ cplx integral_direct(double x, double dt) {
-  if (x == 0.0) return {dt, 0.0};
-  double sn, cs;
-  sincos_cw(0.5 * (x * dt), sn, cs);
-  const double f = 2.0 * sn / x;
-  return {cs * f, sn * f};
-}
-
-__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
-  asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-      : "+d"(c0), "+d"(c1)
-      : "d"(a), "d"(b));
-}
-
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
-  const unsigned s = (unsigned)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem_src));
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N));
-}
-
-// ---- TMA 1-D bulk copy global -> shared, completion signalled on an mbarrier (one thread issues a
-// whole stage: no per-thread address arithmetic, no cp.async bookkeeping in the consumer warps)
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(void* mbar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(mbar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_fence_init() {
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(void* mbar, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(mbar)), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, unsigned bytes, void* mbar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(smem_u32(mbar))
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(void* mbar, unsigned parity) {
-  unsigned ok = 0;
-  const unsigned addr = smem_u32(mbar);
-  while (!ok) {
-    asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                 : "=r"(ok) : "r"(addr), "r"(parity) : "memory");
-  }
-}
-__device__ __forceinline__ void fence_proxy_async() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
 
 __device__ __forceinline__ void pair_from_index(int p, int d, int& m, int& n) {
   m = 0;
@@ -628,10 +512,6 @@ __device__ __forceinline__ void gen_diag(Gen& g, const double* unit_consts, int 
 
 // ---- pair unit (product form): S = I(w + Om) + I(w - Om), D = i (I(w + Om) - I(w - Om)), times phase.
 // Returns true if this lane needs the direct re-evaluation (cancellation in sin((w +- Om) dt / 2)).
-// |x| < SMALL_SIN on the high word only (integer pipe: a DSETP would take an FP64-pipe slot)
-__device__ __forceinline__ int abs_hi(double x) { return __double2hiint(x) & 0x7fffffff; }
-constexpr int SMALL_SIN_HI = 0x3F56A09E;  // high word of 2^-10 sqrt(2)
-
 __device__ __forceinline__ bool pair_values(const Gen& g, double Om, double Ch, double Sh, Vals& v) {
   const double t1 = g.hc * Ch, t3 = g.hs * Ch;
   const double zp_re = fma(-g.hs, Sh, t1), zp_im = fma(g.hc, Sh, t3);  // sqrt2 e^{i (w+Om) dt/2}

@@ -34,6 +34,8 @@
 #include <cstdlib>
 
 #include "ffb_common.cuh"
+#include "ffb_device.cuh"
+#include "ffb_phase.cuh"
 
 namespace {
 
@@ -57,52 +59,6 @@ constexpr int STAGE_BYTES = STAGE_P + STAGE_C;
 constexpr int I8_MAX_CHUNK_STAGES = 1536 / I8_SEGS;  // 1536 segments: 5 pairs x 24576 K entries x 2^14 < 2^31
 constexpr double I8_MAGIC = 6755399441055744.0 + 551911719040.0;  // 1.5 2^52 + sum_i 128 256^i
 
-// ---- math helpers (same formulas and constants as ffb_ctrlmat.cu) ------------------------------------
-__constant__ double SCK[16] = {
-    6.36619772367581382433e-01, 6755399441055744.0, 1.57079632679489655800e+00,
-    6.12323399573676603587e-17, 1.58969099521155010221e-10, -2.50507602534068634195e-08,
-    2.75573137070700676789e-06, -1.98412698298579493134e-04, 8.33333333332248946124e-03,
-    -1.66666666666666324348e-01, -1.13596475577881948265e-11, 2.08757232129817482790e-09,
-    -2.75573143513906633035e-07, 2.48015872894767294178e-05, -1.38888888888741095749e-03,
-    4.16666666666666019037e-02};
-
-__device__ __forceinline__ void sincos_cw(double x, double& sn, double& cs) {
-  double kd = fma(x, SCK[0], SCK[1]);
-  const int q = __double2loint(kd);
-  kd -= SCK[1];
-  double r = fma(-kd, SCK[2], x);
-  r = fma(-kd, SCK[3], r);
-  const double r2 = r * r;
-  double ps = fma(r2, SCK[4], SCK[5]);
-  ps = fma(ps, r2, SCK[6]);
-  ps = fma(ps, r2, SCK[7]);
-  ps = fma(ps, r2, SCK[8]);
-  ps = fma(ps, r2, SCK[9]);
-  const double s = fma(r * r2, ps, r);
-  double pc = fma(r2, SCK[10], SCK[11]);
-  pc = fma(pc, r2, SCK[12]);
-  pc = fma(pc, r2, SCK[13]);
-  pc = fma(pc, r2, SCK[14]);
-  pc = fma(pc, r2, SCK[15]);
-  const double c = fma(r2 * r2, pc, fma(r2, -0.5, 1.0));
-  const double ss = (q & 1) ? c : s;
-  const double cc = (q & 1) ? s : c;
-  const int s_flip = (q & 2) << 30;
-  const int c_flip = ((q + 1) & 2) << 30;
-  sn = __hiloint2double(__double2hiint(ss) ^ s_flip, __double2loint(ss));
-  cs = __hiloint2double(__double2hiint(cc) ^ c_flip, __double2loint(cc));
-}
-
-__device__ __forceinline__ double rcp_nr(double x) {
-  double r;
-  asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(x));
-  double e = fma(-x, r, 1.0);
-  r = fma(r, e, r);
-  e = fma(-x, r, 1.0);
-  r = fma(r, e, r);
-  return r;
-}
-
 // 1 / x to ~2^-46 (seed 2^-23, one Newton step): the operand is cut to 39 bits afterwards, so the second
 // Newton step of rcp_nr would be wasted (12 reciprocals per segment and frequency)
 __device__ __forceinline__ double rcp_nr1(double x) {
@@ -112,47 +68,7 @@ __device__ __forceinline__ double rcp_nr1(double x) {
   return fma(r, e, r);
 }
 
-constexpr double SQRT2 = 1.41421356237309504880;
-constexpr int SMALL_SIN_HI = 0x3F56A09E;  // high word of 2^-10 sqrt(2)
-__device__ __forceinline__ int abs_hi(double x) { return __double2hiint(x) & 0x7fffffff; }
-
-// I(x) = (e^{i x dt} - 1) / (i x) with the rounding sequence of numeric.py:156-165; = dt for x == 0
-__device__ __forceinline__ cplx integral_direct(double x, double dt) {
-  if (x == 0.0) return {dt, 0.0};
-  double sn, cs;
-  sincos_cw(0.5 * (x * dt), sn, cs);
-  const double f = 2.0 * sn / x;
-  return {cs * f, sn * f};
-}
-
-// ---- PTX wrappers ------------------------------------------------------------------------------------
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(void* mbar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(mbar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(void* mbar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(mbar)) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(void* mbar, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(mbar)), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(void* mbar, unsigned parity) {
-  unsigned ok = 0;
-  const unsigned addr = smem_u32(mbar);
-  while (!ok) {
-    asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                 : "=r"(ok) : "r"(addr), "r"(parity) : "memory");
-  }
-}
-__device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, unsigned bytes, void* mbar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(smem_u32(mbar))
-               : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
+// ---- tcgen05 wrappers --------------------------------------------------------------------------------
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
@@ -414,7 +330,7 @@ __global__ void __launch_bounds__(I8_THREADS, 1) ctrlmat_i8_kernel(const I8Param
       mbar_init(&bar_empty[s], 1);
     }
     mbar_init(&bar_done, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_fence_init();
   }
   if (warp == I8_GEN_WARPS) {  // the producer warp owns the tensor memory
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(&tmem_base_s)));

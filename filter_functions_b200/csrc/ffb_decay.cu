@@ -19,14 +19,9 @@
 // The frequency axis is cut into chunks (grid.x) whose partial sums are reduced in a fixed order by
 // reduce_kernel (deterministic, no atomics), which also applies the 1 / (2 pi).
 #include "ffb_common.cuh"
+#include "ffb_device.cuh"
 
 namespace {
-
-__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
-  asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-      : "+d"(c0), "+d"(c1)
-      : "d"(a), "d"(b));
-}
 
 // WS[s, w] = u_w S[s, w]: trapezoid weight times spectrum (complex if the spectrum is)
 __global__ void __launch_bounds__(256)

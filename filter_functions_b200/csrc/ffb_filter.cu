@@ -11,6 +11,7 @@
 #include <cstdlib>
 
 #include "ffb_common.cuh"
+#include "ffb_device.cuh"
 #include "ffb_peer.cuh"
 
 namespace {
@@ -73,14 +74,6 @@ ff_fidelity_kernel(int P, int n_nops, int n_basis, int n_omega, size_t ld,
 constexpr int GRAM_W = 16;       // frequencies per CTA
 constexpr int GRAM_KC = 8;       // basis elements per stage (4 per half-warp)
 __host__ __device__ constexpr int gram_stages(bool tri) { return tri ? 4 : 3; }   // pairs of panels: 64 KB per stage
-
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)),
-               "l"(gmem_src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 // acc[i][j] += conj(x_i) y_j for the basis elements kk = 2 m + half of one stage
 template <int TL, bool DIAG, bool WHOLE>
