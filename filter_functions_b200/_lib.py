@@ -280,7 +280,8 @@ class DispatchRecord(ctypes.Structure):
     """``ffb_dispatch_record`` of include/ffb200.h."""
     _fields_ = [('kernel', ctypes.c_char*64), ('prologue', ctypes.c_char*96)] + [
         (name, c_int) for name in ('S', 'passes_per_chunk', 'n_pass', 'n_sp', 'pps', 'transposed', 'n_rb',
-                                   'n_wtiles', 'ctas_by_regs', 'block', 'n_blocks', 'n_omega')]
+                                   'n_wtiles', 'ctas_by_regs', 'block', 'n_blocks', 'n_omega', 'route',
+                                   'chunk_segs', 'n_bands', 'n_proxies')]
 
 
 def dispatch_log(ctx=None):

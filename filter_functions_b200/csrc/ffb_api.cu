@@ -286,6 +286,7 @@ void ffb_destroy(ffb_ctx* ctx) {
   for (auto& kv : ctx->host_free_blocks) cudaFreeHost(kv.second);
   for (auto& kv : ctx->host_live_blocks) cudaFreeHost(kv.first);
   if (ctx->trig_table) cudaFree(ctx->trig_table);
+  if (ctx->band_counts) cudaFree(ctx->band_counts);
   if (ctx->stage_host) cudaFreeHost(ctx->stage_host);
   if (ctx->stage_out) cudaFreeHost(ctx->stage_out);
   if (ctx->conv_dev) cudaFree(ctx->conv_dev);
@@ -376,6 +377,20 @@ int copy_log(std::deque<ffb_dispatch_record>& log, ffb_dispatch_record* out, int
 
 int ffb_dispatch_log(ffb_ctx* ctx, ffb_dispatch_record* out, int capacity) {
   if (!ctx) return FFB_EINVAL;
+  // banded blocks: the plan kernel counted their bands on the device (n_bands = -(ring slot + 1) until read)
+  bool pending = false;
+  for (const auto& rec : ctx->dispatch_log) pending = pending || rec.n_bands < 0;
+  if (pending && out) {
+    std::vector<int> counts((size_t)2 * FFB_DISPATCH_LOG_MAX);
+    FFB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    FFB_CUDA(ctx, cudaMemcpy(counts.data(), ctx->band_counts, counts.size() * sizeof(int), cudaMemcpyDeviceToHost));
+    for (auto& rec : ctx->dispatch_log) {
+      if (rec.n_bands >= 0) continue;
+      const int slot = -rec.n_bands - 1;
+      rec.n_bands = counts[2 * slot];
+      rec.n_proxies = counts[2 * slot + 1];
+    }
+  }
   return copy_log(ctx->dispatch_log, out, capacity);
 }
 

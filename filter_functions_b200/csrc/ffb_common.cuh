@@ -60,6 +60,10 @@ struct ffb_ctx {
   int64_t launches = 0;
   // 256-entry table of (sin, cos)(k pi / 128) for the table-driven sincos of the control-matrix kernels
   double* trig_table = nullptr;
+  // bands and proxies of the last FFB_DISPATCH_LOG_MAX banded control-matrix blocks, written by the plan
+  // kernel; ffb_dispatch_log reads them into the records
+  int* band_counts = nullptr;
+  unsigned band_counts_next = 0;
   // second stream for bulk host<->device copies that overlap kernels (the pulse pipeline, the control
   // matrix, ffb_concatenate_pulses); ordered against `stream` with the two events
   cudaStream_t copy_stream = nullptr;

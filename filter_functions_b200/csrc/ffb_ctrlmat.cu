@@ -274,6 +274,15 @@ transform_small_kernel(int G, int n_nops, int n_basis, int parts_j, int parts_k,
                          n_coeffs, basis, dst);
 }
 
+// Centre of chunk c of L segments.  On the banded route (see band_eval_kernel) the stream carries the segment
+// start times relative to the centre of their chunk, so that the partial sum of a chunk is a smooth function
+// of omega of exponential type T_c / 2; the evaluation kernel puts e^{i w t_c} back with the same t_c.
+__device__ __forceinline__ double chunk_centre(const double* __restrict__ t, const double* __restrict__ dt,
+                                               int G, int L, int c) {
+  const int g0 = c * L, g1 = min(G, g0 + L) - 1;
+  return 0.5 * (t[g0] + (t[g1] + dt[g1]));
+}
+
 // ------------------------------------------------------------------------------------------------
 // prologue 2: the operand stream of the main kernel.
 // Per row block rb and pass (4 consecutive segments) the stream holds 1 + n_pairs units:
@@ -327,7 +336,7 @@ __host__ __device__ inline StreamGeom make_geom(int rows, int G, int d, int MT) 
 template <bool STAGED>
 __global__ void __launch_bounds__(256)
 assemble_kernel(StreamGeom geo, int G, int d, int rows, int n_jrows, int n_krows, int split_rf,
-                const double* __restrict__ Bbar_g, const double* __restrict__ Cbar_g,
+                int chunk_segs, const double* __restrict__ Bbar_g, const double* __restrict__ Cbar_g,
                 const double* __restrict__ eigvals, const double* __restrict__ dt,
                 const double* __restrict__ t, double* __restrict__ stream) {
   extern __shared__ __align__(16) double stage[];
@@ -407,7 +416,8 @@ assemble_kernel(StreamGeom geo, int G, int d, int rows, int n_jrows, int n_krows
     if (e < 8) {
       const int which = e >> 2, slot = e & 3;
       const int g = geo.transposed ? pass : g0 + slot;
-      if (g < G) val = which == 0 ? t[g] : dt[g];
+      if (g < G) val = which == 0 ? t[g] - (chunk_segs ? chunk_centre(t, dt, G, chunk_segs, g / chunk_segs) : 0.0)
+                                  : dt[g];
       out[col + e] = val;
     } else {
       const int u = 1 + (e - 8) / 12, c = (e - 8) % 12;
@@ -442,6 +452,7 @@ struct MainParams {
   const double* stream;
   const double* omega;
   double* partial;  // [S][rows_pad][n_omega] complex
+  const int* n_live;  // banded route: frequency slots [*n_live, n_omega) are unused (nullptr: all used)
   int n_omega;
   int rows_pad;     // n_rb * MT * 8
   int n_pass;
@@ -590,6 +601,7 @@ template <int MT, int NW>
 __global__ void __launch_bounds__(NW * 32, (MT <= 2 ? 3 : MT >= 10 ? 3 : 1))
 ctrlmat_main_kernel(const MainParams p) {
   extern __shared__ __align__(16) double smem[];
+  if (p.n_live && (int)blockIdx.x * NW * 8 >= __ldg(p.n_live)) return;  // whole CTA past the used slots
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
   const int q = lane & 3;
@@ -902,6 +914,7 @@ template <int MT, int NW, int NP, int NSP, bool SPLIT = false>
 __global__ void __launch_bounds__(NW * 32, (MT <= 2 ? 3 : MT >= 10 ? 3 : 1))
 ctrlmat_static_kernel(const MainParams p) {
   extern __shared__ __align__(16) double smem[];
+  if (p.n_live && (int)blockIdx.x * NW * 8 >= __ldg(p.n_live)) return;  // whole CTA past the used slots
   constexpr int NU = 1 + NP;
   constexpr int DIAG_UNIT = MT * 32 + 8, PAIR_UNIT = 2 * MT * 32 + 12;
   const int lane = threadIdx.x & 31;
@@ -1444,20 +1457,270 @@ finalize_kernel(int S, int rows_pad, int n_nops, int n_basis, int parts_j, int p
 }
 
 // ------------------------------------------------------------------------------------------------
+// banded route: Chebyshev interpolation of per-chunk partial sums on dense frequency bands (DESIGN 4.1.1)
+//
+// With the segments cut into chunks c of at most T_c and the stream's times taken relative to the chunk
+// centres t_c (assemble_kernel, chunk_segs > 0), the main kernel's partial sum of chunk c is
+//     Z_c(w) = e^{-i w t_c} B^(c)(w) = int_{|s| <= T_c/2} e^{i w s} f(t_c + s) ds,
+// an entire function of exponential type T_c / 2.  On a band [k W, (k + 1) W) of width W = 4 sigma / T_c its
+// Chebyshev coefficients beyond degree p are bounded by 2 |J_p(sigma)| ||f||_1, so the values at the
+// BAND_P Chebyshev points of the second kind determine Z_c on the band to rounding level (BAND_P = 48,
+// sigma = 16: max_{p >= 48} |J_p(16)| = 4.8e-19).  A band whose targets outnumber its proxies by the rule
+// in band_plan_kernel is evaluated as
+//     B(w) = sum_c e^{i w t_c} sum_p l_p(w) Z_c(w_p),
+// every other frequency directly, B(w) = sum_c e^{i w t_c} Z_c(w).
+// ------------------------------------------------------------------------------------------------
+constexpr int BAND_P = 48;
+constexpr double BAND_SIGMA = 16.0;
+constexpr int BAND_MIN_G = 1024;       // shorter pulses: too few segments per chunk for the route to pay
+constexpr int BAND_CHUNK_QUANTUM = 128;  // chunk length: a multiple of this many segments
+constexpr int BAND_PLAN_THREADS = 1024;
+constexpr int BAND_EVAL_OUTS = 8;      // (j, k) outputs per thread of band_eval_kernel
+
+struct BandPlan {
+  double* eval_omega;  // [n] frequencies the main kernel evaluates: proxies and direct targets, then 1.0
+  int* target;         // [n] slot of a direct target, -(run + 1) of an interpolated one
+  int* run_start;      // [n + 1] first target of each run of targets in one band
+  int* run_base;       // [n] first slot of a run (its proxies if it pays, else its direct targets)
+  int* counts;         // [3] used slots, interpolated bands, proxies
+  int* log_counts;     // [2] bands and proxies for the dispatch record
+};
+
+__device__ __forceinline__ double band_of(double w, double W) { return floor(w / W); }
+__device__ __forceinline__ bool band_pays(int len, double r_cost) { return len * (1.0 - r_cost) > BAND_P; }
+
+// exclusive prefix sum over the block (blockDim.x == BAND_PLAN_THREADS); *total = sum over the block
+__device__ int block_exclusive_scan(int v, int* total) {
+  __shared__ int warp_sums[32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int incl = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int u = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += u;
+  }
+  if (lane == 31) warp_sums[warp] = incl;
+  __syncthreads();
+  if (warp == 0) {
+    int s = warp_sums[lane];
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int u = __shfl_up_sync(0xffffffffu, s, o);
+      if (lane >= o) s += u;
+    }
+    warp_sums[lane] = s;
+  }
+  __syncthreads();
+  const int before = (warp ? warp_sums[warp - 1] : 0) + incl - v;
+  *total = warp_sums[31];
+  __syncthreads();
+  return before;
+}
+
+// One CTA: splits the frequency block into runs of consecutive targets that share a band of the global
+// lattice [k W, (k + 1) W), decides per run whether interpolation pays, and writes the compacted list of
+// frequencies the main kernel evaluates.  Enqueue-only: omega, t and dt stay on the device.
+// r_cost = evaluation cost of an interpolated target in units of a direct one; a run of len targets pays
+// when len (1 - r_cost) > BAND_P.
+__global__ void __launch_bounds__(BAND_PLAN_THREADS)
+band_plan_kernel(const double* __restrict__ omega, int n, const double* __restrict__ t,
+                 const double* __restrict__ dt, int G, int L, int S, double r_cost, BandPlan plan) {
+  __shared__ double tc_max[32];
+  __shared__ double s_W;
+  const int tid = threadIdx.x;
+  // ---- longest chunk -> band width
+  double dur = 0.0;
+  for (int c = tid; c < S; c += blockDim.x) {
+    const int g0 = c * L, g1 = min(G, g0 + L) - 1;
+    dur = fmax(dur, (t[g1] + dt[g1]) - t[g0]);
+  }
+  for (int o = 16; o; o >>= 1) dur = fmax(dur, __shfl_xor_sync(0xffffffffu, dur, o));
+  if ((tid & 31) == 0) tc_max[tid >> 5] = dur;
+  __syncthreads();
+  if (tid == 0) {
+    double m = 0.0;
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) m = fmax(m, tc_max[w]);
+    s_W = 4.0 * BAND_SIGMA / m;
+  }
+  __syncthreads();
+  const double W = s_W;
+  // ---- runs: target i starts a run when its band differs from that of target i - 1
+  int n_runs = 0;
+  for (int i0 = 0; i0 < n; i0 += blockDim.x) {
+    const int i = i0 + tid;
+    int flag = 0;
+    if (i < n) flag = (i == 0 || band_of(omega[i], W) != band_of(omega[i - 1], W)) ? 1 : 0;
+    int tile_runs;
+    const int before = block_exclusive_scan(flag, &tile_runs);
+    if (i < n) {
+      const int run = n_runs + before + flag - 1;
+      plan.target[i] = run;  // run index for now
+      if (flag) plan.run_start[run] = i;
+    }
+    n_runs += tile_runs;
+  }
+  if (tid == 0) plan.run_start[n_runs] = n;
+  __syncthreads();
+  // ---- slots per run: BAND_P proxies if it pays, else its targets
+  int n_slots = 0, n_bands = 0;
+  for (int r0 = 0; r0 < n_runs; r0 += blockDim.x) {
+    const int r = r0 + tid;
+    int slots = 0, pays = 0;
+    if (r < n_runs) {
+      const int len = plan.run_start[r + 1] - plan.run_start[r];
+      pays = band_pays(len, r_cost) ? 1 : 0;
+      slots = pays ? BAND_P : len;
+    }
+    int tile_slots, tile_bands;
+    const int base = block_exclusive_scan(slots, &tile_slots);
+    block_exclusive_scan(pays, &tile_bands);
+    if (r < n_runs) plan.run_base[r] = n_slots + base;
+    n_slots += tile_slots;
+    n_bands += tile_bands;
+  }
+  __syncthreads();
+  // ---- targets and proxies
+  for (int i = tid; i < n; i += blockDim.x) {
+    const int r = plan.target[i];
+    const int s0 = plan.run_start[r];
+    if (band_pays(plan.run_start[r + 1] - s0, r_cost)) {
+      plan.target[i] = -(r + 1);
+      if (i - s0 < BAND_P) {  // proxy i - s0 of the run (a paying run has more than BAND_P targets)
+        const int j = i - s0;
+        const double h = 0.5 * W, c = (band_of(omega[s0], W) + 0.5) * W;
+        plan.eval_omega[plan.run_base[r] + j] = fma(h, cospi((double)j / (BAND_P - 1)), c);
+      }
+    } else {
+      const int slot = plan.run_base[r] + (i - s0);
+      plan.target[i] = slot;
+      plan.eval_omega[slot] = omega[i];
+    }
+  }
+  for (int i = n_slots + tid; i < n; i += blockDim.x) plan.eval_omega[i] = 1.0;
+  if (tid == 0) {
+    plan.counts[0] = n_slots;
+    plan.counts[1] = n_bands;
+    plan.counts[2] = n_bands * BAND_P;
+    plan.log_counts[0] = n_bands;
+    plan.log_counts[1] = n_bands * BAND_P;
+  }
+}
+
+// Replaces finalize_kernel on the banded route.  Thread = one target x BAND_EVAL_OUTS outputs (j, k):
+//   out[j, k, w] = sum_c e^{i w t_c} sum_{pj, pk} i^{pj + pk} Zhat_c[row(j, k, pj, pk)](w)
+// with Zhat_c(w) = partial_c(slot of w) for a direct target and sum_p l_p(w) partial_c(proxy p) for an
+// interpolated one (barycentric weights of the second kind, real; a target on a proxy takes its value).
+// Fixed summation order, no atomics: a second call repeats every bit.
+__global__ void __launch_bounds__(128)
+band_eval_kernel(int n, int S, int L, int G, int rows_pad, int n_nops, int n_basis, int parts_j,
+                 int parts_k, size_t ld_out, int split_rf, const double* __restrict__ omega,
+                 const double* __restrict__ t, const double* __restrict__ dt, BandPlan plan,
+                 const double* __restrict__ partial, double* __restrict__ out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int n_out = n_nops * n_basis;
+  const int jk0 = blockIdx.y * BAND_EVAL_OUTS;
+  const int n_krows = n_basis * parts_k;
+  const size_t n_slots = (size_t)n;
+  const double w = omega[i];
+  const int tg = plan.target[i];
+  int base;
+  double l[BAND_P];
+  if (tg >= 0) {
+    base = tg;
+  } else {
+    const int r = -tg - 1;
+    base = plan.run_base[r];
+    const double* nodes = plan.eval_omega + base;
+    int hit = -1;
+#pragma unroll
+    for (int p = 0; p < BAND_P; ++p) hit = nodes[p] == w ? p : hit;
+    if (hit >= 0) {
+#pragma unroll
+      for (int p = 0; p < BAND_P; ++p) l[p] = p == hit ? 1.0 : 0.0;
+    } else {
+      // barycentric formula in the evaluated node frequencies themselves (it is invariant under the affine
+      // map to [-1, 1]); weights (-1)^p, halved at the two ends
+      double sum = 0.0;
+#pragma unroll
+      for (int p = 0; p < BAND_P; ++p) {
+        const double wp = (p == 0 || p == BAND_P - 1) ? 0.5 : 1.0;
+        const double q = ((p & 1) ? -wp : wp) / (w - nodes[p]);
+        l[p] = q;
+        sum += q;
+      }
+      const double inv = 1.0 / sum;
+#pragma unroll
+      for (int p = 0; p < BAND_P; ++p) l[p] *= inv;
+    }
+  }
+  double acc_re[BAND_EVAL_OUTS], acc_im[BAND_EVAL_OUTS];
+#pragma unroll
+  for (int o = 0; o < BAND_EVAL_OUTS; ++o) acc_re[o] = acc_im[o] = 0.0;
+  const double2* part = reinterpret_cast<const double2*>(partial);
+  for (int c = 0; c < S; ++c) {
+    double sn, cs;
+    sincos(w * chunk_centre(t, dt, G, L, c), &sn, &cs);
+#pragma unroll
+    for (int o = 0; o < BAND_EVAL_OUTS; ++o) {
+      const int jk = jk0 + o;
+      if (jk >= n_out) break;
+      const int j = jk / n_basis, k = jk % n_basis;
+      double re = 0.0, im = 0.0;
+      for (int pj = 0; pj < parts_j; ++pj) {
+        for (int pk = 0; pk < parts_k; ++pk) {
+          int row = (j * parts_j + pj) * n_krows + k * parts_k + pk;
+          if (split_rf > 0) row = k == 0 ? split_rf + j : j * (n_basis - 1) + k - 1;
+          const double2* src = part + ((size_t)c * rows_pad + row) * n_slots + base;
+          double zr, zi;
+          if (tg >= 0) {
+            const double2 z = src[0];
+            zr = z.x;
+            zi = z.y;
+          } else {
+            zr = 0.0;
+            zi = 0.0;
+#pragma unroll
+            for (int p = 0; p < BAND_P; ++p) {
+              const double2 z = src[p];
+              zr = fma(l[p], z.x, zr);
+              zi = fma(l[p], z.y, zi);
+            }
+          }
+          switch ((pj + pk) & 3) {  // multiply by i^(pj+pk)
+            case 0: re += zr; im += zi; break;
+            case 1: re -= zi; im += zr; break;
+            default: re -= zr; im -= zi; break;
+          }
+        }
+      }
+      acc_re[o] = fma(cs, re, fma(-sn, im, acc_re[o]));
+      acc_im[o] = fma(cs, im, fma(sn, re, acc_im[o]));
+    }
+  }
+#pragma unroll
+  for (int o = 0; o < BAND_EVAL_OUTS; ++o) {
+    const int jk = jk0 + o;
+    if (jk < n_out) reinterpret_cast<double2*>(out)[(size_t)jk * ld_out + i] = make_double2(acc_re[o], acc_im[o]);
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 // launch plumbing
 // ------------------------------------------------------------------------------------------------
 constexpr int STAGE_TARGET_BYTES = 32 * 1024;
 constexpr int STAGE_MAX_BYTES = 48 * 1024;
 
 template <int MT, int NW>
-int launch_main(ffb_ctx* ctx, MainParams p, int n_wtiles, int n_rb, int S, ffb_dispatch_record& disp) {
+int launch_main(ffb_ctx* ctx, MainParams p, int n_wtiles, int n_rb, int S, ffb_dispatch_record& disp,
+                bool timed) {
   auto kern = ctrlmat_main_kernel<MT, NW>;
   snprintf(disp.kernel, sizeof disp.kernel, "ctrlmat_main_kernel<%d, %d>", MT, NW);
   const size_t smem = (size_t)2 * p.stage_doubles * sizeof(double);
   FFB_TRY(ffb_func_smem(ctx, kern, smem));
   dim3 grid(n_wtiles, n_rb, S);
   int slot = -1;
-  FFB_TRY(ffb_time_begin(ctx, &slot));
+  if (timed) FFB_TRY(ffb_time_begin(ctx, &slot));
   kern<<<grid, NW * 32, smem, ctx->stream>>>(p);
   FFB_LAUNCHED(ctx);
   FFB_TRY(ffb_time_end(ctx, slot));
@@ -1465,7 +1728,8 @@ int launch_main(ffb_ctx* ctx, MainParams p, int n_wtiles, int n_rb, int S, ffb_d
 }
 
 template <int MT, int NW, int NP, int NSP, bool SPLIT = false>
-int launch_static(ffb_ctx* ctx, MainParams p, int n_wtiles, int n_rb, int S, ffb_dispatch_record& disp) {
+int launch_static(ffb_ctx* ctx, MainParams p, int n_wtiles, int n_rb, int S, ffb_dispatch_record& disp,
+                  bool timed) {
   auto kern = ctrlmat_static_kernel<MT, NW, NP, NSP, SPLIT>;
   snprintf(disp.kernel, sizeof disp.kernel, "ctrlmat_static_kernel<%d, %d, %d, %d, %s>", MT, NW, NP, NSP,
            SPLIT ? "true" : "false");
@@ -1473,7 +1737,7 @@ int launch_static(ffb_ctx* ctx, MainParams p, int n_wtiles, int n_rb, int S, ffb
   FFB_TRY(ffb_func_smem(ctx, kern, smem));
   dim3 grid(n_wtiles, n_rb, S);
   int slot = -1;
-  FFB_TRY(ffb_time_begin(ctx, &slot));
+  if (timed) FFB_TRY(ffb_time_begin(ctx, &slot));
   kern<<<grid, NW * 32, smem, ctx->stream>>>(p);
   FFB_LAUNCHED(ctx);
   FFB_TRY(ffb_time_end(ctx, slot));
@@ -1573,7 +1837,20 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
                       parts_k == 1 && n_basis == 16 && n_nops == 6 && MT == 12 && geo.n_rb == 1 && !geo.transposed;
   if (const char* e = getenv("FFB_CTRLMAT_SPLIT_IDENTITY")) split_tensor = split_tensor && atoi(e) != 0;
   const int split_t = split_tensor ? n_nops * (n_basis - 1) : 0;
-  DevBuf Bbar, Cbar, stream, partial, i8_scales;
+  // block boundaries on multiples of 64 frequencies (the frequency tiles of all kernel variants)
+  const int n_blocks = blocks ? std::max(1, std::min(blocks->n_blocks, ceil_div(n_omega_all, 64))) : 1;
+  const int per_block = ceil_div(ceil_div(n_omega_all, n_blocks), 64) * 64;
+  // banded route (DESIGN 4.1.1): tensor path in the regular layout, long pulses, blocks that can hold a band
+  // worth interpolating.  Chunks of band_L segments, the shortest multiple of BAND_CHUNK_QUANTUM (doubled) whose
+  // partials [S][rows_pad][per_block] stay within 1 GiB.
+  const bool banded = !use_dfma && !use_i8 && !geo.transposed && d >= 2 && G >= BAND_MIN_G &&
+                      std::min(per_block, n_omega_all) > BAND_P;
+  int band_L = 0;
+  if (banded) {
+    band_L = BAND_CHUNK_QUANTUM;
+    while (band_L < G && (size_t)ceil_div(G, band_L) * rows_pad * per_block * 16 > ((size_t)1 << 30)) band_L *= 2;
+  }
+  DevBuf Bbar, Cbar, stream, partial, i8_scales, plan_buf;
   std::string prologue;  // for the dispatch record
   if (!fused_prologue) {
     FFB_TRY(Bbar.alloc(ctx, (size_t)G * n_jrows * dd * 16));
@@ -1644,12 +1921,12 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
     if (stage_bytes <= 96 * 1024) {
       FFB_TRY(ffb_func_smem(ctx, assemble_kernel<true>, stage_bytes));
       assemble_kernel<true><<<blocks, 256, stage_bytes, ctx->stream>>>(
-          geo, G, d, rows, n_jrows, n_krows, split_t, Bbar.as<double>(), Cbar.as<double>(), eigvals, dt, t,
+          geo, G, d, rows, n_jrows, n_krows, split_t, band_L, Bbar.as<double>(), Cbar.as<double>(), eigvals, dt, t,
           stream.as<double>());
       prologue += "+assemble_kernel<true>";
     } else {
       assemble_kernel<false><<<blocks, 256, 0, ctx->stream>>>(
-          geo, G, d, rows, n_jrows, n_krows, split_t, Bbar.as<double>(), Cbar.as<double>(), eigvals, dt, t,
+          geo, G, d, rows, n_jrows, n_krows, split_t, band_L, Bbar.as<double>(), Cbar.as<double>(), eigvals, dt, t,
           stream.as<double>());
       prologue += "+assemble_kernel<false>";
     }
@@ -1822,9 +2099,9 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
   long long s_cap = (long long)geo.n_pass / min_passes;
   s_cap = std::min(s_cap, 64 * slots / base_ctas + 1);
   s_cap = std::min(s_cap, (long long)(((size_t)1 << 30) / ((size_t)rows_pad * n_omega * 16)) + 1);
-  const int S_max = (int)std::max<long long>(1, s_cap);
+  const int S_max = banded ? 0 : (int)std::max<long long>(1, s_cap);
   const double overhead_passes = 2.0;
-  int S = 1, ppc = geo.n_pass;
+  int S = banded ? ceil_div(G, band_L) : 1, ppc = banded ? band_L / 4 : geo.n_pass;
   double best_cost = 1e300;
   for (int s = 1; s <= S_max; ++s) {
     int c = ceil_div(geo.n_pass, s);
@@ -1842,6 +2119,32 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
 
   FFB_TRY(partial.alloc(ctx, (size_t)S * rows_pad * n_omega * 16));
   p.partial = partial.as<double>();
+  p.n_live = nullptr;
+  BandPlan plan = {};
+  int stage_slot = -1;  // the banded route times plan, main kernel and evaluation as one stage
+  if (banded) {
+    const size_t n = (size_t)n_omega;
+    FFB_TRY(plan_buf.alloc(ctx, n * sizeof(double) + (4 * n + 4) * sizeof(int)));
+    plan.eval_omega = plan_buf.as<double>();
+    plan.target = reinterpret_cast<int*>(plan.eval_omega + n);
+    plan.run_start = plan.target + n;
+    plan.run_base = plan.run_start + n + 1;
+    plan.counts = plan.run_base + n;
+    if (!ctx->band_counts)
+      FFB_CUDA(ctx, cudaMalloc(&ctx->band_counts, (size_t)2 * FFB_DISPATCH_LOG_MAX * sizeof(int)));
+    const int log_slot = (int)(ctx->band_counts_next++ % FFB_DISPATCH_LOG_MAX);
+    plan.log_counts = ctx->band_counts + 2 * log_slot;
+    disp.route = 1;
+    disp.chunk_segs = band_L;
+    disp.n_bands = -(log_slot + 1);  // filled from the device by ffb_dispatch_log
+    // an interpolated target costs S (2 P + 4) real multiply-adds per row, a direct one 2 (1 + d (d - 1)) G
+    const double r_cost = (double)S * (2 * BAND_P + 4) / (2.0 * (1 + d * (d - 1)) * G);
+    FFB_TRY(ffb_time_begin(ctx, &stage_slot));
+    band_plan_kernel<<<1, BAND_PLAN_THREADS, 0, ctx->stream>>>(omega, n_omega, t, dt, G, band_L, S, r_cost, plan);
+    FFB_LAUNCHED(ctx);
+    p.omega = plan.eval_omega;
+    p.n_live = plan.counts;
+  }
 
   // d = 4 (6 level pairs), one pass per stage or a pass in two pieces: statically scheduled variant
   bool use_static = geo.n_pairs == 6 && !geo.transposed && p.pps == 1 && p.n_sp <= 2 &&
@@ -1866,29 +2169,36 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
   disp.n_wtiles = n_wtiles;
   disp.ctas_by_regs = ctas_by_regs;
   if (use_static16) {
-    FFB_TRY((launch_static<12, 4, 30, 7>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    FFB_TRY((launch_static<12, 4, 30, 7>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
   } else if (use_static8) {
-    if (MT == 12 && p.n_sp == 5) FFB_TRY((launch_static<12, 4, 28, 5>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else if (MT == 12 && p.n_sp == 6) FFB_TRY((launch_static<12, 4, 28, 6>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else if (MT == 12) FFB_TRY((launch_static<12, 4, 28, 7>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else if (p.n_sp == 4) FFB_TRY((launch_static<8, 4, 28, 4>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else if (p.n_sp == 5) FFB_TRY((launch_static<8, 4, 28, 5>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else FFB_TRY((launch_static<8, 4, 28, 6>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    if (MT == 12 && p.n_sp == 5) FFB_TRY((launch_static<12, 4, 28, 5>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else if (MT == 12 && p.n_sp == 6) FFB_TRY((launch_static<12, 4, 28, 6>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else if (MT == 12) FFB_TRY((launch_static<12, 4, 28, 7>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else if (p.n_sp == 4) FFB_TRY((launch_static<8, 4, 28, 4>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else if (p.n_sp == 5) FFB_TRY((launch_static<8, 4, 28, 5>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else FFB_TRY((launch_static<8, 4, 28, 6>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
   } else if (use_static) {
-    if (MT == 12 && p.n_sp == 2 && split_t) FFB_TRY((launch_static<12, 4, 6, 2, true>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else if (MT == 12 && p.n_sp == 2) FFB_TRY((launch_static<12, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else if (MT == 12) FFB_TRY((launch_static<12, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else if (MT == 10 && p.n_sp == 2) FFB_TRY((launch_static<10, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else if (MT == 10) FFB_TRY((launch_static<10, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else if (MT == 8 && p.n_sp == 2) FFB_TRY((launch_static<8, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else if (MT == 8) FFB_TRY((launch_static<8, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else if (p.n_sp == 2) FFB_TRY((launch_static<6, 8, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
-    else FFB_TRY((launch_static<6, 8, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp)));
+    if (MT == 12 && p.n_sp == 2 && split_t) FFB_TRY((launch_static<12, 4, 6, 2, true>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else if (MT == 12 && p.n_sp == 2) FFB_TRY((launch_static<12, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else if (MT == 12) FFB_TRY((launch_static<12, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else if (MT == 10 && p.n_sp == 2) FFB_TRY((launch_static<10, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else if (MT == 10) FFB_TRY((launch_static<10, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else if (MT == 8 && p.n_sp == 2) FFB_TRY((launch_static<8, 4, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else if (MT == 8) FFB_TRY((launch_static<8, 4, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else if (p.n_sp == 2) FFB_TRY((launch_static<6, 8, 6, 2>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
+    else FFB_TRY((launch_static<6, 8, 6, 1>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded)));
   } else {
-    FFB_DISPATCH_MT(MT, FFB_TRY((launch_main<MT_, NW_>(ctx, p, n_wtiles, geo.n_rb, S, disp))));
+    FFB_DISPATCH_MT(MT, FFB_TRY((launch_main<MT_, NW_>(ctx, p, n_wtiles, geo.n_rb, S, disp, !banded))));
   }
 
-  {
+  if (banded) {
+    const dim3 grid(ceil_div(n_omega, 128), ceil_div(n_nops * n_basis, BAND_EVAL_OUTS));
+    band_eval_kernel<<<grid, 128, 0, ctx->stream>>>(n_omega, S, band_L, G, rows_pad, n_nops, n_basis, parts_j,
+                                                    parts_k, ld_out, split_t, omega, t, dt, plan,
+                                                    partial.as<double>(), out);
+    FFB_LAUNCHED(ctx);
+    FFB_TRY(ffb_time_end(ctx, stage_slot));
+  } else {
     const size_t total = (size_t)n_nops * n_basis * n_omega;
     const unsigned blocks = (unsigned)std::min<size_t>(ceil_div_sz(total, 256), (size_t)ctx->sm_count * 16);
     finalize_kernel<<<blocks, 256, 0, ctx->stream>>>(S, rows_pad, n_nops, n_basis, parts_j, parts_k,
@@ -1898,9 +2208,6 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
   return FFB_OK;
   };  // run_block
 
-  // block boundaries on multiples of 64 frequencies (the frequency tiles of all kernel variants)
-  const int n_blocks = blocks ? std::max(1, std::min(blocks->n_blocks, ceil_div(n_omega_all, 64))) : 1;
-  const int per_block = ceil_div(ceil_div(n_omega_all, n_blocks), 64) * 64;
   const bool trace = ffb_trace();
   for (int w0 = 0; w0 < n_omega_all; w0 += per_block) {
     const int w1 = std::min(n_omega_all, w0 + per_block);
@@ -1915,10 +2222,11 @@ int ffbi_control_matrix(ffb_ctx* ctx, int G, int d, int n_nops, int n_basis, int
     if (trace)
       fprintf(stderr,
               "[ffb trace] control matrix G %d d %d rows %d, block %d/%d (%d frequencies): %s after %s; S %d "
-              "passes_per_chunk %d n_pass %d n_sp %d pps %d transposed %d n_rb %d n_wtiles %d ctas_by_regs %d\n",
+              "passes_per_chunk %d n_pass %d n_sp %d pps %d transposed %d n_rb %d n_wtiles %d ctas_by_regs %d "
+              "route %d chunk_segs %d\n",
               G, d, rows, disp.block + 1, disp.n_blocks, disp.n_omega, disp.kernel, disp.prologue, disp.S,
               disp.passes_per_chunk, disp.n_pass, disp.n_sp, disp.pps, disp.transposed, disp.n_rb, disp.n_wtiles,
-              disp.ctas_by_regs);
+              disp.ctas_by_regs, disp.route, disp.chunk_segs);
     if (blocks && blocks->after_block) FFB_TRY(blocks->after_block(w0, w1));
   }
   return FFB_OK;

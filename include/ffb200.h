@@ -360,8 +360,9 @@ int ffb_shadow_query(ffb_ctx* ctx, const void* host, size_t bytes);
 int ffb_shadow_drop(ffb_ctx* ctx, const void* host, size_t bytes);
 int ffb_shadow_stats(ffb_ctx* ctx, int* count, size_t* bytes, int64_t* hits, size_t* hit_bytes);
 
-/* Kernel-level timing of the control-matrix main kernel: average duration (ms) of the launches of
- * the dominant kernel recorded with CUDA events on the launching stream since the last reset. */
+/* Kernel-level timing of the control-matrix stage: total duration (ms) and number of the timed launches,
+ * recorded with CUDA events on the launching stream since the last reset.  A timed launch is the main
+ * kernel, or on the banded route the plan, main and evaluation kernels of a frequency block together. */
 int ffb_kernel_timing_enable(ffb_ctx* ctx, int enable);
 int ffb_kernel_timing_read(ffb_ctx* ctx, double* total_ms, int64_t* launches, int reset);
 
@@ -395,6 +396,11 @@ typedef struct {
   int ctas_by_regs;      /* resident CTAs per SM the registers allow (sets the stage budget) */
   int block, n_blocks;   /* this frequency block and the number of blocks of the call */
   int n_omega;           /* frequencies in this block */
+  int route;             /* 0: every frequency evaluated directly; 1: banded (Chebyshev interpolation of
+                            per-chunk partial sums on dense bands, DESIGN 4.1.1) */
+  int chunk_segs;        /* banded: segments per chunk L (S = ceil(G / L) chunks); else 0 */
+  int n_bands;           /* banded: bands interpolated in this block; else 0 */
+  int n_proxies;         /* banded: proxy frequencies evaluated for them (BAND_P per band); else 0 */
 } ffb_dispatch_record;
 int ffb_dispatch_log(ffb_ctx* ctx, ffb_dispatch_record* out, int capacity);
 int ffb_diag_dispatch_log(ffb_ctx* ctx, ffb_dispatch_record* out, int capacity);
